@@ -38,7 +38,7 @@ L2_FLUSH_BYTES = 256 << 20
 def parse_args():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=50)
+    p.add_argument("--steps", type=int, help="timed steps of c2 and of the reference arm (default 50)")
     p.add_argument("--warmup", type=int, default=5)
     p.add_argument("--impl", default="ours", choices=["ours", "reference"])
     p.add_argument("--hypotheses", type=int, default=64, help="hypotheses per GPU (weak scaling)")
@@ -61,7 +61,18 @@ def parse_args():
                    help="c2 (default) is the configuration the metric is quoted on and the only one with the "
                         "full contract line; c1 / c3 / c4 / c5 run BASELINE.json's other configurations "
                         "(scripts/gpu_configs.py, scripts/gpu_sweep.py) and print their result as one line")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="c2: write what the last timed step computed (rank 0) as DIR/<name>.npy, float32; "
+                        "see dump_outputs()")
+    args = p.parse_args()
+    if args.steps is not None and args.impl == "ours" and args.workload != "c2":
+        p.error("--steps applies to c2 and to --impl reference; c1 / c3 / c4 / c5 time their scripts' own counts")
+    args.steps = 50 if args.steps is None else args.steps
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        p.error("--dump-outputs needs --impl ours --workload c2")
+    return args
 
 
 def workload_name(B):
@@ -155,6 +166,31 @@ def ncu_traffic(kernel):
             return json.load(f)[kernel]["dram_bytes_per_launch"]
     except Exception:
         return None
+
+
+DUMP_SAMPLE = 1 << 22  # elements kept of a larger output (depth: 19.7 M, grad_sdf: 16.8 M at 64 hypotheses)
+DUMP_LIMIT = 64_000_000  # bytes written by one dump
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each array of `outputs` (name -> array) as out_dir/<name>.npy in float32, so that two builds
+    can be compared output for output.  An array of more than DUMP_SAMPLE elements is written as the 1-D
+    array of its elements at DUMP_SAMPLE flat indices drawn without replacement by numpy's
+    default_rng(0), in ascending index order: the same positions in every run with the same arguments."""
+    import numpy as np
+
+    arrays = {}
+    for name, a in outputs.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        arrays[name] = a
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the limit of {DUMP_LIMIT}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -264,9 +300,8 @@ def run_reference_arm(args, rank):
     if rank != 0:
         return
     # the arm's own config: every step renders ALL hypotheses of the workload (64 x 640x480 is ~0.25 s of
-    # CPU work per step on 16 threads); steps / warm-up as given (same floor of 3 warm-up steps as the GPU
-    # arm), bounded only so that an accidental --steps 100000 still ends
-    steps = max(1, min(args.steps, 400))
+    # CPU work per step on 16 threads); steps / warm-up as given (same floor of 3 warm-up steps as the GPU arm)
+    steps = args.steps
     warmup = max(args.warmup, 3)
     sample = args.hypotheses
     mpix, ms, cores = time_cpu(sample, steps, warmup)
@@ -595,6 +630,11 @@ def main():
     with ClockSampler(local_rank) as clocks:
         launches["kernels"] = launches["steps"] = 0
         total_ms = timed(step, K, Wm, finish=drain if distributed else None)
+    if args.dump_outputs and rank == 0:  # before the launches below overwrite the step's outputs
+        dump_outputs(args.dump_outputs, {
+            "depth": depth.cpu().numpy(), "loss_sum": sums[0].cpu().numpy(), "n_overlap": sums[1].cpu().numpy(),
+            "grad_sdf": g_sdf.cpu().numpy(), "grad_position": g_pos.cpu().numpy(),
+            "grad_orientation": g_quat.cpu().numpy(), "grad_inv_scale": g_is.cpu().numpy()})
     kernels_timed = launches["kernels"] * K // (K + Wm)  # warm-up steps launch the same kernels
     if distributed:
         t = torch.tensor([total_ms], device=dev)

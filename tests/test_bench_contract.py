@@ -95,3 +95,21 @@ def test_reference_arm_line():
         assert d["cpu_baseline"]["value"] == d["value"] and d["cpu_baseline"]["kind"] in ("reference", "port")
         if pattern.startswith("r02"):
             assert d["config"] == bench.config_object(d["config"]["hypotheses_per_gpu"], False)
+
+
+def test_dump_outputs_writes_float32_and_samples_large_outputs_at_fixed_positions(tmp_path):
+    import numpy as np
+    import pytest
+
+    big = np.arange(bench.DUMP_SAMPLE + 1000, dtype=np.float64)  # values = flat indices
+    small = np.ones((4, 3), np.float32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"big": big, "small": small})
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_SAMPLE,) and np.array_equal(a, b)
+    assert (np.diff(a) > 0).all() and a[-1] <= big[-1]  # distinct positions, in index order
+    s = np.load(tmp_path / "a" / "small.npy")
+    assert s.dtype == np.float32 and np.array_equal(s, small)
+    with pytest.raises(SystemExit):  # over the size limit: nothing is written
+        bench.dump_outputs(str(tmp_path / "c"), {f"x{i}": big for i in range(4)})
+    assert not (tmp_path / "c").exists()

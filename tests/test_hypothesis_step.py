@@ -640,7 +640,7 @@ def test_fused_optimizer_on_a_device_that_is_not_current(cuda_device):
     CURRENT device's stream and never calls cudaSetDevice, so the Python side must make it current) and
     give the results of the same optimiser built on cuda:0."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     torch.cuda.set_device(0)
     a = _make_optimizers(torch.device("cuda:0"), 4, True, "fused")
     b = _make_optimizers(torch.device("cuda:1"), 4, True, "fused")
