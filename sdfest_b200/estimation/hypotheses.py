@@ -19,7 +19,7 @@ from .. import _lib
 from ..differentiable_renderer import Camera, render_and_compare
 from ..differentiable_renderer.sdf_renderer import (_camera_params, _grid_operand, _ptr,
                                                     _skewed_elems, _stream)
-from . import losses
+from . import losses, views
 from .decoder import FusedTailDecoder
 from .fused import decode_render_compare
 
@@ -159,7 +159,6 @@ class HypothesisOptimizer:
         self.sdf_grad_mode = get_sdf_grad_mode()
         self.lrs, self.betas, self.eps = tuple(float(x) for x in lrs), tuple(betas), float(eps)
         self.camera, self.threshold, self.group = camera, float(threshold), group
-        self.depth_obs = depth_obs.contiguous()
         self.depth_weight, self.pc_weight = depth_weight, pc_weight
         self.position = position.detach().clone().requires_grad_(True)
         self.orientation = orientation.detach().clone().requires_grad_(True)
@@ -176,55 +175,10 @@ class HypothesisOptimizer:
         if self.optimizer_impl == "torch":
             self.optimizer = torch.optim.Adam(groups, betas=self.betas, eps=self.eps,
                                               capturable=self.position.is_cuda)
-        # observed points, once (the only host syncs), sub-sampled to a fixed size
         B = self.position.shape[0]
-        self.point_counts = None  # (B,) points hypothesis b owns, when the clouds differ
-        self._views = None
-        self.point_capacity, self._n_points, self.max_points = int(point_capacity), None, int(max_points)
-        if point_capacity and (self.optimizer_impl != "fused" or (not multiview and self.depth_obs.dim() != 2)):
+        self.point_capacity, self.max_points = int(point_capacity), int(max_points)
+        if point_capacity and (self.optimizer_impl != "fused" or (not multiview and depth_obs.dim() != 2)):
             raise ValueError("point_capacity needs the fused path and one shared observation (H,W) or views (V,H,W)")
-        if multiview:
-            V = int(camera_positions.shape[0])
-            if instance is not None:
-                raise ValueError("views and object instances cannot be combined")
-            if tuple(camera_positions.shape) != (V, 3) or tuple(camera_orientations.shape) != (V, 4) \
-                    or self.depth_obs.dim() != 3 or self.depth_obs.shape[0] != V:
-                raise ValueError("camera_positions (V,3), camera_orientations (V,4) and depth_obs (V,H,W) expected")
-            dev_o = self.depth_obs.device
-            self._views = (camera_positions.detach().to(dev_o, torch.float32).contiguous(),
-                           camera_orientations.detach().to(dev_o, torch.float32).contiguous())
-            self._view_points = [losses.subsample_points(losses.depth_to_pointcloud(d, camera), max_points)
-                                 for d in self.depth_obs]
-            self._view_counts = [int(p.shape[0]) for p in self._view_points]
-            if point_capacity:
-                # fixed-size clouds (padding outside every volume) and private copies of what reset() overwrites
-                self.depth_obs = self.depth_obs.clone()
-                self._views = tuple(t.clone() for t in self._views)
-                self._view_points = [self._padded_cloud(p, int(point_capacity)) for p in self._view_points]
-            self.points = self._view_points[0]
-        elif self.depth_obs.dim() == 2:
-            if instance is not None:
-                raise ValueError("`instance` needs one observed depth map per object instance (K,H,W)")
-            self.points = losses.subsample_points(losses.depth_to_pointcloud(self.depth_obs, camera),
-                                                  max_points)
-            if point_capacity:
-                self.depth_obs = self.depth_obs.clone()  # reset() overwrites it: never the caller's tensor
-                self._load_points(self.points, int(point_capacity))
-        else:
-            # object instances: hypothesis b is compared with the depth map and the points of instance
-            # instance[b] (default: one map per hypothesis)
-            if instance is None:
-                instance = torch.arange(B, device=self.depth_obs.device)
-            instance = instance.to(device=self.depth_obs.device, dtype=torch.int64)
-            if instance.shape != (B,) or self.depth_obs.dim() != 3:
-                raise ValueError("depth_obs (K,H,W) and instance (B,) expected")
-            if int(instance.min()) < 0 or int(instance.max()) >= self.depth_obs.shape[0]:
-                raise ValueError("instance index out of range")
-            clouds, counts = losses.depth_to_pointclouds(self.depth_obs, camera, max_points)
-            self.points = clouds.index_select(0, instance).contiguous()
-            self.point_counts = counts.index_select(0, instance)
-            self.depth_obs = self.depth_obs.index_select(0, instance).contiguous()
-        self.instance = instance
         self.last_losses = None
         self.inlier_threshold = None if inlier_threshold is None else float(inlier_threshold)
         if self.inlier_threshold is not None:
@@ -238,63 +192,109 @@ class HypothesisOptimizer:
             self.best_scale = self.scale.detach().clone()
             self.best_latent = None if self.latent is None else self.latent.detach().clone()
             self._iteration = torch.zeros(B, dtype=torch.int32, device=dev0)  # optimizer="torch" (device-side: survives graph replay)
-            # valid pixels depend on the observation alone (simple_setup.py:186): counted once
-            if self.optimizer_impl == "fused" and self.inlier_threshold <= 1.0 and not multiview:  # else: sdfr_inlier_count recounts both
-                n_valid = (self.depth_obs != 0).flatten(-2).sum(-1).to(torch.float32)
-                self._inl[1].copy_(n_valid.expand(B) if n_valid.dim() == 0 else n_valid)
+        # valid pixels depend on the observation alone (simple_setup.py:186): counted once where the fused iteration
+        # counts inliers only (thresholds <= 1, no views); else sdfr_inlier_count recounts both every iteration
+        self._valid_once = self.optimizer_impl == "fused" and self.inlier_threshold is not None \
+            and self.inlier_threshold <= 1.0 and not multiview
+        self.depth_obs = self._views = self.instance = self._n_points = None
+        self.point_counts = None  # (B,) points hypothesis b owns, when the clouds differ
+        self._set_observation(depth_obs, camera_positions, camera_orientations, instance)
         self._graph = None
         self._shard_sizes = None  # exchanged on the first gather of run()
         if self.optimizer_impl == "fused":
             with torch.cuda.device(self.position.device):
                 self._init_fused()
 
-    @staticmethod
-    def _padded_cloud(points: torch.Tensor, capacity: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """(M,3) observed points in a (capacity,3) buffer, the rest far outside every SDF volume."""
-        n = int(points.shape[0])
-        if n > capacity:
-            raise ValueError(f"{n} observed points exceed point_capacity {capacity}")
-        if out is None:
-            out = torch.empty((capacity, 3), dtype=torch.float32, device=points.device)
-        out.fill_(losses.PAD_COORDINATE)
-        out[:n].copy_(points)
-        return out
+    def _set_observation(self, depth_obs: torch.Tensor, camera_positions: Optional[torch.Tensor] = None,
+                         camera_orientations: Optional[torch.Tensor] = None,
+                         instance: Optional[torch.Tensor] = None) -> None:
+        """The observation into the buffers every iteration reads: depth images and camera poses, each view's
+        observed points (one shared observation is one view), sub-sampled once -- the only host syncs --, the
+        weight pc_weight / (true number of points) per hypothesis in device memory, and the valid pixels where
+        they are counted once.  Construction allocates the buffers (private copies: never the caller's tensors);
+        reset() overwrites them in place, so a captured graph keeps reading them, and raises before it writes any.
 
-    def _load_points(self, points: torch.Tensor, capacity: int) -> None:
-        """Observed points (M,3) into the fixed-size buffer (allocated on first use)."""
-        n = int(points.shape[0])
-        if n > capacity:
-            raise ValueError(f"{n} observed points exceed point_capacity {capacity}")
-        if self.points is None or self.points.shape[0] != capacity:
-            self.points = torch.empty((capacity, 3), dtype=torch.float32, device=points.device)
-        self.points.fill_(losses.PAD_COORDINATE)
-        self.points[:n].copy_(points)
-        self._n_points = n
-
-    def _reset_views(self, depth_obs: torch.Tensor, camera_positions: Optional[torch.Tensor],
-                     camera_orientations: Optional[torch.Tensor]) -> None:
-        """New observations (V,H,W) and camera poses of the view loop into the buffers the captured graph reads."""
-        if tuple(depth_obs.shape) != tuple(self.depth_obs.shape):
-            raise ValueError("depth_obs must keep its shape (V,H,W)")
-        if self.pc_weight and not self.point_capacity:
-            raise RuntimeError("new observations need point_capacity (the cloud sizes are baked in)")
-        clouds = []
-        if self.pc_weight:
-            clouds = [losses.subsample_points(losses.depth_to_pointcloud(d, self.camera), self.max_points)
-                      for d in depth_obs]
-            for c in clouds:  # before any buffer is touched: may raise
-                if int(c.shape[0]) > self.point_capacity:
-                    raise ValueError(f"{int(c.shape[0])} observed points exceed point_capacity {self.point_capacity}")
-        for v, c in enumerate(clouds):
-            self._padded_cloud(c, self.point_capacity, out=self._view_points[v])
-            n = int(c.shape[0])
-            self._view_counts[v] = n
-            self._view_up_p[v].fill_(self.pc_weight / n if n else 0.0)
-        self.depth_obs.copy_(depth_obs)
-        if camera_positions is not None:
-            self._views[0].copy_(camera_positions.reshape(self._views[0].shape))
-        if camera_orientations is not None:
-            self._views[1].copy_(camera_orientations.reshape(self._views[1].shape))
+        Object instances (construction only): ``depth_obs`` (K,H,W) and ``instance`` (B,): hypothesis b is compared
+        with the depth map and the points of instance[b] (default: one map per hypothesis)."""
+        B, cap, first = int(self.position.shape[0]), self.point_capacity, self.depth_obs is None
+        views = camera_positions is not None or self._views is not None
+        if first:
+            if views:
+                if instance is not None:
+                    raise ValueError("views and object instances cannot be combined")
+                V = int(camera_positions.shape[0])
+                if tuple(camera_positions.shape) != (V, 3) or tuple(camera_orientations.shape) != (V, 4) \
+                        or depth_obs.dim() != 3 or depth_obs.shape[0] != V:
+                    raise ValueError("camera_positions (V,3), camera_orientations (V,4) and depth_obs (V,H,W) expected")
+            elif depth_obs.dim() == 2:
+                if instance is not None:
+                    raise ValueError("`instance` needs one observed depth map per object instance (K,H,W)")
+            else:
+                if instance is None:
+                    instance = torch.arange(B, device=depth_obs.device)
+                instance = instance.to(device=depth_obs.device, dtype=torch.int64)
+                if instance.shape != (B,) or depth_obs.dim() != 3:
+                    raise ValueError("depth_obs (K,H,W) and instance (B,) expected")
+                if int(instance.min()) < 0 or int(instance.max()) >= depth_obs.shape[0]:
+                    raise ValueError("instance index out of range")
+            W, H = int(self.camera.width), int(self.camera.height)
+            if self.optimizer_impl == "fused" and tuple(depth_obs.shape[-2:]) != (H, W):
+                raise RuntimeError(f"depth_obs must have shape (V,{H},{W})" if views
+                                   else f"depth_obs must have shape ({H},{W}) or ({B},{H},{W})")
+        else:
+            if tuple(depth_obs.shape) != tuple(self.depth_obs.shape):
+                raise ValueError(f"depth_obs must keep its shape {tuple(self.depth_obs.shape)}")
+            if self.pc_weight and not cap:
+                raise RuntimeError("a new observation needs point_capacity (the cloud sizes are baked in)")
+        if instance is not None:
+            clouds, counts = losses.depth_to_pointclouds(depth_obs, self.camera, self.max_points)
+            self.instance = instance
+            self.points = clouds.index_select(0, instance).contiguous()
+            self.point_counts = counts.index_select(0, instance)
+            self.depth_obs = depth_obs.index_select(0, instance).contiguous()
+            # hypothesis b weighs its own points with pc_weight / counts[b]
+            n = self.point_counts.to(torch.float32)
+            self._up_p = torch.where(n > 0, self.pc_weight / n.clamp(min=1.0), torch.zeros_like(n)).contiguous()
+        else:
+            V = int(depth_obs.shape[0]) if views else 1
+            poses = [None if p is None else p.detach().reshape(V, k)
+                     for p, k in ((camera_positions, 3), (camera_orientations, 4))]
+            clouds = []
+            if first or self.pc_weight:
+                clouds = [losses.subsample_points(losses.depth_to_pointcloud(d, self.camera), self.max_points)
+                          for d in (depth_obs if views else depth_obs[None])]
+            for c in clouds:
+                if cap and int(c.shape[0]) > cap:
+                    raise ValueError(f"{int(c.shape[0])} observed points exceed point_capacity {cap}")
+            if first:
+                dev = self.position.device
+                self.depth_obs = torch.empty_like(depth_obs, memory_format=torch.contiguous_format)
+                # with point_capacity: fixed-size clouds, padded outside every volume (point loss exactly 0 there)
+                self._view_points = [torch.empty((cap, 3), dtype=torch.float32, device=c.device) if cap else c
+                                     for c in clouds]
+                self._view_counts = [0] * V
+                self._view_up_p = [torch.empty((B,), dtype=torch.float32, device=dev) for _ in range(V)]
+                self.points = self._view_points[0]
+                if views:
+                    self._views = tuple(torch.empty((V, k), dtype=torch.float32, device=depth_obs.device)
+                                        for k in (3, 4))
+                else:
+                    self._up_p = self._view_up_p[0]
+            self.depth_obs.copy_(depth_obs)
+            for v, c in enumerate(clouds):
+                n = int(c.shape[0])
+                if cap:
+                    self._view_points[v].fill_(losses.PAD_COORDINATE)
+                    self._view_points[v][:n].copy_(c)
+                self._view_counts[v] = n
+                self._view_up_p[v].fill_(self.pc_weight / n if n else 0.0)
+            if not views:
+                self._n_points = self._view_counts[0]  # true number of points of the shared cloud
+            for buf, p in zip(self._views or (), poses):
+                if p is not None:
+                    buf.copy_(p)
+        if self._valid_once:
+            self._inl[1].copy_((self.depth_obs != 0).flatten(-2).sum(-1))
 
     def reset(self, position: torch.Tensor, orientation: torch.Tensor, scale: torch.Tensor,
               latent: Optional[torch.Tensor] = None, depth_obs: Optional[torch.Tensor] = None,
@@ -312,28 +312,17 @@ class HypothesisOptimizer:
             raise RuntimeError("reset() supports one shared observation or views (no object instances)")
         if not self._V and (camera_positions is not None or camera_orientations is not None):
             raise ValueError("camera poses can only be reset on an optimiser constructed with views")
+        if self.latent is not None and latent is None:
+            raise ValueError("latent expected")
         with torch.no_grad(), torch.cuda.device(self.position.device):
-            if self._V:
-                if depth_obs is not None:
-                    self._reset_views(depth_obs, camera_positions, camera_orientations)
-                elif camera_positions is not None or camera_orientations is not None:
-                    self._reset_views(self.depth_obs.clone(), camera_positions, camera_orientations)
-            elif depth_obs is not None:
-                if tuple(depth_obs.shape) != tuple(self.depth_obs.shape):
-                    raise ValueError("depth_obs must keep its shape")
-                if self._M and not self.point_capacity:
-                    raise RuntimeError("a new observation needs point_capacity (the cloud size is baked in)")
-                if self._M:
-                    pts = losses.subsample_points(losses.depth_to_pointcloud(depth_obs, self.camera), self.max_points)
-                    self._load_points(pts, self.point_capacity)  # before any buffer is touched: may raise
-                    self._up_p.fill_((self.pc_weight / self._n_points) if self._n_points else 0.0)
-                self.depth_obs.copy_(depth_obs)
+            if depth_obs is not None or camera_positions is not None or camera_orientations is not None:
+                # new camera poses alone: the clouds are reloaded from the current observation
+                self._set_observation(self.depth_obs if depth_obs is None else depth_obs, camera_positions,
+                                      camera_orientations)
             self.position.copy_(position.reshape(self.position.shape))
             self.orientation.copy_(orientation.reshape(self.orientation.shape))
             self.scale.copy_(scale.reshape(self.scale.shape))
             if self.latent is not None:
-                if latent is None:
-                    raise ValueError("latent expected")
                 self.latent.copy_(latent.reshape(self.latent.shape))
             for t in (self._m, self._v, self._t, self._small, self._loss):
                 t.zero_()
@@ -341,13 +330,13 @@ class HypothesisOptimizer:
                 self._g_raw.zero_()
                 self._loss_extra.zero_()
             if self.inlier_threshold is not None:
-                self._inl.zero_()
+                self._inl[0].zero_()
+                if not self._valid_once:  # else: the valid pixels of the observation, counted by _set_observation
+                    self._inl[1].zero_()
                 self.inlier_ratio.zero_()
                 self.best_inlier_ratio.fill_(-1.0)
                 self.best_iteration.fill_(-1)
                 self._iteration.zero_()
-                if self.inlier_threshold <= 1.0 and not self._V:  # views recount both every iteration
-                    self._inl[1].fill_(float((self.depth_obs != 0).sum()))
             self._hyp_step(_lib.STEP_NO_UPDATE)  # unit quaternions and 1/scale of the new estimate
         self.last_losses = None
 
@@ -368,16 +357,7 @@ class HypothesisOptimizer:
         W, H = int(self.camera.width), int(self.camera.height)
         V = 0 if self._views is None else int(self.depth_obs.shape[0])
         self._V = V
-        if V:
-            if tuple(self.depth_obs.shape[1:]) != (H, W):
-                raise RuntimeError(f"depth_obs must have shape (V,{H},{W})")
-            self._obs_stride = 0
-        elif tuple(self.depth_obs.shape) == (H, W):
-            self._obs_stride = 0
-        elif tuple(self.depth_obs.shape) == (B, H, W):
-            self._obs_stride = H * W
-        else:
-            raise RuntimeError(f"depth_obs must have shape ({H},{W}) or ({B},{H},{W})")
+        self._obs_stride = 0 if self.point_counts is None else H * W  # (B,H,W): one image per hypothesis
         # every small per-hypothesis buffer in one allocation: consumed AND cleared by the step kernel
         # (with views: [V,B,...] each, consumed and cleared by sdfr_views_pull_back)
         NB = max(V, 1) * B
@@ -418,30 +398,14 @@ class HypothesisOptimizer:
             pb = torch.zeros(8 * B, dtype=torch.float32, device=dev)
             self._pb = (pb[:3 * B], pb[3 * B:7 * B], pb[7 * B:])
             self._view_M = [int(p.shape[0]) if self.pc_weight else 0 for p in self._view_points]
-            self._view_points = [p.contiguous() for p in self._view_points]
-            # the weight pc_weight / (true number of points of the view) lives in device memory: reset() can
-            # change it under a captured graph (with point_capacity the buffers are larger than the clouds)
-            self._view_up_p = [torch.full((B,), self.pc_weight / n if (n and m) else 0.0, dtype=torch.float32,
-                                          device=dev) for n, m in zip(self._view_counts, self._view_M)]
         self._M = M
-        if self.point_capacity:
-            # fixed-size buffer: the weight pc_weight / (true count) lives in device memory (upstream and,
-            # with SDFR_LOSS_WEIGHTED, the loss), so reset() can change it under a captured graph
-            self._points_stride, self._point_flags = 0, _lib.LOSS_WEIGHTED
-            self._point_weight = 1.0
-            n = self._n_points
-            self._up_p = torch.full((B,), (self.pc_weight / n) if n else 0.0, dtype=torch.float32, device=dev)
-        elif self.point_counts is None:
-            self._points_stride, self._point_flags = 0, 0
-            self._point_weight = (self.pc_weight / M) if M else 0.0
-            self._up_p = torch.full((B,), self._point_weight, dtype=torch.float32, device=dev)
-        else:
-            # per-instance clouds: hypothesis b weighs its own points with pc_weight / counts[b], in
-            # the gradients (upstream) and -- SDFR_LOSS_WEIGHTED -- in the loss sum itself
-            self._points_stride, self._point_flags = 3 * M, _lib.LOSS_WEIGHTED
-            self._point_weight = 1.0
-            n = self.point_counts.to(torch.float32)
-            self._up_p = torch.where(n > 0, self.pc_weight / n.clamp(min=1.0), torch.zeros_like(n)).contiguous()
+        # fixed-size and per-instance clouds: the weight pc_weight / (true count) lives in device memory (_up_p:
+        # upstream and, with SDFR_LOSS_WEIGHTED, the loss), so reset() can change it under a captured graph;
+        # a plain shared cloud passes it to the step kernel as a scalar
+        weighted = bool(self.point_capacity) or self.point_counts is not None
+        self._point_flags = _lib.LOSS_WEIGHTED if weighted else 0
+        self._point_weight = 1.0 if weighted else ((self.pc_weight / M) if M else 0.0)
+        self._points_stride = 0 if self.point_counts is None else 3 * M
         self._up_d = torch.full((B,), float(self.depth_weight), dtype=torch.float32, device=dev)
         if self.decoder is None:
             sdf = self.sdf.contiguous()
@@ -533,6 +497,47 @@ class HypothesisOptimizer:
             self.point_constraint[2], self._g_raw.data_ptr(), self._loss_extra.data_ptr(), _stream()),
             "sdfr_point_constraint")
 
+    def _tail_forward(self, with_bounds: bool):
+        """The decoder trunk on a fresh latent leaf (autograd graph: latent -> x only), then the tail into this
+        iteration's grids; ``with_bounds``: the tail also compares every value with the hypothesis' hit-threshold
+        bound as it stores it, so the empty-space bounds cost no extra read of the grids.  Returns (leaf, x, w)."""
+        dec, B, R = self.decoder, self.position.shape[0], self._R
+        grids, gstride, layout = self._grid_op
+        leaf = self._latent_leaf()
+        x = dec.trunk(leaf).contiguous()
+        w, bias = dec.tail_parameters()
+        args = (x.data_ptr(), int(x.shape[1]), int(x.shape[2]), w.data_ptr(), _ptr(bias), _ptr(dec.base), B, R,
+                grids.data_ptr(), gstride, layout)
+        if with_bounds:
+            _lib.check(_lib.lib().sdfr_decoder_tail_forward_bounds(
+                *args, self.position.data_ptr(), self._inv_scale.data_ptr(), self.threshold,
+                self._bounds.data_ptr(), _stream()), "sdfr_decoder_tail_forward_bounds")
+        else:
+            _lib.check(_lib.lib().sdfr_decoder_tail_forward(*args, _stream()), "sdfr_decoder_tail_forward")
+        return leaf, x, w
+
+    def _tail_backward(self, leaf: torch.Tensor, x: torch.Tensor, w: torch.Tensor, n_overlap=None, upstream=None,
+                       g_sdf_pc=None, g_sdf_pc_stride: int = 0) -> torch.Tensor:
+        """Tail adjoint of the gradient grid(s) -- with ``n_overlap`` and ``upstream`` it also applies the deferred
+        depth-loss normalisation -- then autograd through the trunk: the latent gradient."""
+        B, R = self.position.shape[0], self._R
+        g_x = torch.empty_like(x)
+        _lib.check(_lib.lib().sdfr_decoder_tail_backward(
+            self._g_sdf.data_ptr(), R ** 3, n_overlap, upstream, g_sdf_pc, g_sdf_pc_stride, w.data_ptr(),
+            int(x.shape[1]), int(x.shape[2]), B, R, g_x.data_ptr(), _stream()), "sdfr_decoder_tail_backward")
+        (g_latent,) = torch.autograd.grad(x, leaf, g_x)
+        return g_latent.contiguous()
+
+    def _track_best(self, flags: int) -> None:
+        """sdfr_track_best: inlier ratio of this iteration's counts, and the best estimate so far."""
+        _lib.check(_lib.lib().sdfr_track_best(
+            self._inl[0].data_ptr(), self._inl[1].data_ptr(), self.position.data_ptr(),
+            self.orientation.data_ptr(), self.scale.data_ptr(), _ptr(self.latent), self._L, self.position.shape[0],
+            self._t.data_ptr(), self.inlier_ratio.data_ptr(), self.best_inlier_ratio.data_ptr(),
+            self.best_iteration.data_ptr(), self.best_position.data_ptr(),
+            self.best_orientation.data_ptr(), self.best_scale.data_ptr(), _ptr(self.best_latent),
+            flags, _stream()), "sdfr_track_best")
+
     def _fused_views_iteration(self) -> torch.Tensor:
         """One iteration over V views of the same object (simple_setup.py:408-463) as C-ABI launches:
         decoder tail -> camera-frame poses -> per view {bounds, render + compare, its backward with the
@@ -541,17 +546,10 @@ class HypothesisOptimizer:
         B, R, V = self.position.shape[0], self._R, self._V
         W, H, cx, cy, fx, fy = _camera_params(self.camera)
         grids, gstride, layout = self._grid_op
-        dec, x = self.decoder, None
         flags = _lib.GRAD_POSITION | _lib.GRAD_ORIENTATION | _lib.GRAD_INV_SCALE
-        if dec is not None:
+        if self.decoder is not None:
             self._g_both.zero_()
-            leaf = self._latent_leaf()
-            x = dec.trunk(leaf).contiguous()
-            w, bias = dec.tail_parameters()
-            C, S = int(x.shape[1]), int(x.shape[2])
-            _lib.check(lib.sdfr_decoder_tail_forward(
-                x.data_ptr(), C, S, w.data_ptr(), _ptr(bias), _ptr(dec.base), B, R, grids.data_ptr(),
-                gstride, layout, _stream()), "sdfr_decoder_tail_forward")
+            leaf, x, w = self._tail_forward(with_bounds=False)
             flags |= _lib.GRAD_SDF
         render_flags = flags | (_lib.SDF_GRAD_EXACT if self.sdf_grad_mode == "exact" else 0)
         cam_p, cam_q = self._views
@@ -599,23 +597,10 @@ class HypothesisOptimizer:
             g_p.data_ptr(), g_q.data_ptr(), g_s.data_ptr(), self._loss_extra.data_ptr(),
             _lib.STEP_CLEAR_INPUTS, _stream()), "sdfr_views_pull_back")
         self._constraint_launch()
-        g_latent = None
-        if dec is not None:
-            g_x = torch.empty_like(x)
-            _lib.check(lib.sdfr_decoder_tail_backward(
-                g_sdf, R ** 3, None, None, None, 0, w.data_ptr(), C, S, B, R, g_x.data_ptr(), _stream()),
-                "sdfr_decoder_tail_backward")
-            (g_latent,) = torch.autograd.grad(x, leaf, g_x)
-            g_latent = g_latent.contiguous()
+        g_latent = None if self.decoder is None else self._tail_backward(leaf, x, w)
         self._hyp_step(_lib.STEP_CLEAR_INPUTS, g_latent, self._g_raw, self._loss_extra)
         if self.inlier_threshold is not None:
-            _lib.check(lib.sdfr_track_best(
-                self._inl[0].data_ptr(), self._inl[1].data_ptr(), self.position.data_ptr(),
-                self.orientation.data_ptr(), self.scale.data_ptr(), _ptr(self.latent), self._L, B,
-                self._t.data_ptr(), self.inlier_ratio.data_ptr(), self.best_inlier_ratio.data_ptr(),
-                self.best_iteration.data_ptr(), self.best_position.data_ptr(),
-                self.best_orientation.data_ptr(), self.best_scale.data_ptr(), _ptr(self.best_latent),
-                _lib.STEP_CLEAR_INPUTS, _stream()), "sdfr_track_best")
+            self._track_best(_lib.STEP_CLEAR_INPUTS)
         self.last_losses = self._loss
         return self.last_losses
 
@@ -626,7 +611,7 @@ class HypothesisOptimizer:
         B, R, M = self.position.shape[0], self._R, self._M
         W, H, cx, cy, fx, fy = _camera_params(self.camera)
         grids, gstride, layout = self._grid_op
-        dec, x, tail_bounds = self.decoder, None, None
+        dec, tail_bounds = self.decoder, None
         main, side = torch.cuda.current_stream(), self._side
 
         def on_side(fn):
@@ -643,22 +628,9 @@ class HypothesisOptimizer:
 
         if dec is not None:
             on_side(clear_grids)
-            leaf = self._latent_leaf()
-            x = dec.trunk(leaf).contiguous()  # autograd graph: latent -> x only
-            w, bias = dec.tail_parameters()
-            C, S = int(x.shape[1]), int(x.shape[2])
+            leaf, x, w = self._tail_forward(with_bounds=self._bounds is not None)
             if self._bounds is not None:
-                # the tail compares every value with the hypothesis' hit-threshold bound as it stores it:
-                # the empty-space bounds cost no extra read of the grids
-                _lib.check(lib.sdfr_decoder_tail_forward_bounds(
-                    x.data_ptr(), C, S, w.data_ptr(), _ptr(bias), _ptr(dec.base), B, R, grids.data_ptr(),
-                    gstride, layout, self.position.data_ptr(), self._inv_scale.data_ptr(), self.threshold,
-                    self._bounds.data_ptr(), _stream()), "sdfr_decoder_tail_forward_bounds")
                 tail_bounds = self._bounds.data_ptr()
-            else:
-                _lib.check(lib.sdfr_decoder_tail_forward(
-                    x.data_ptr(), C, S, w.data_ptr(), _ptr(bias), _ptr(dec.base), B, R, grids.data_ptr(),
-                    gstride, layout, _stream()), "sdfr_decoder_tail_forward")
             if side is not None:
                 main.wait_stream(side)
         flags = _lib.GRAD_POSITION | _lib.GRAD_ORIENTATION | _lib.GRAD_INV_SCALE
@@ -714,67 +686,85 @@ class HypothesisOptimizer:
             on_side(count_inliers)
         g_latent = None
         if dec is not None:
-            g_x = torch.empty_like(x)
-            _lib.check(lib.sdfr_decoder_tail_backward(
-                self._g_sdf.data_ptr(), R ** 3, b["n_overlap"].data_ptr(), self._up_d.data_ptr(),
-                _ptr(self._g_sdf_pc), R ** 3, w.data_ptr(), C, S, B, R, g_x.data_ptr(), _stream()),
-                "sdfr_decoder_tail_backward")
-            (g_latent,) = torch.autograd.grad(x, leaf, g_x)
-            g_latent = g_latent.contiguous()
+            g_latent = self._tail_backward(leaf, x, w, b["n_overlap"].data_ptr(), self._up_d.data_ptr(),
+                                           _ptr(self._g_sdf_pc), R ** 3)
         self._hyp_step(_lib.STEP_CLEAR_INPUTS, g_latent, self._g_raw, self._loss_extra)
         if self.inlier_threshold is not None:
             if side is not None and not inl_fused:
                 main.wait_stream(side)
-            _lib.check(lib.sdfr_track_best(
-                self._inl[0].data_ptr(), self._inl[1].data_ptr(), self.position.data_ptr(),
-                self.orientation.data_ptr(), self.scale.data_ptr(), _ptr(self.latent), self._L, B,
-                self._t.data_ptr(), self.inlier_ratio.data_ptr(), self.best_inlier_ratio.data_ptr(),
-                self.best_iteration.data_ptr(), self.best_position.data_ptr(),
-                self.best_orientation.data_ptr(), self.best_scale.data_ptr(), _ptr(self.best_latent),
-                _lib.STEP_CLEAR_INPUTS | (_lib.TRACK_KEEP_VALID if inl_fused else 0), _stream()),
-                "sdfr_track_best")
+            self._track_best(_lib.STEP_CLEAR_INPUTS | (_lib.TRACK_KEEP_VALID if inl_fused else 0))
         self.last_losses = self._loss
         return self.last_losses
 
-    def _constraint_loss(self):
-        """weight * point_constraint_loss on the un-normalised orientation (simple_setup.py:164-175)."""
-        if self.point_constraint is None:
-            return 0.0
-        from . import views
+    # ------------------------------------------------------------------------------------
+    # optimizer="torch": the package's autograd operators and torch.optim.Adam
+    # ------------------------------------------------------------------------------------
+    def _torch_loss(self, q: torch.Tensor):
+        """(loss, rendered depth, the observation the inlier ratio compares it with, no-overlap mask) of the
+        current parameters; ``q`` is the unit orientation."""
+        if self._views is not None:
+            # V views of the same object (simple_setup.py:420-462): the pose is moved into every camera frame,
+            # every view is rendered, compared and scored against its own observed points, the losses are
+            # summed; autograd carries the gradients back through the rigid maps
+            grids = self._grids()
+            grids4 = grids if grids.dim() == 4 else grids[None]
+            position_c, orientation_c = views.to_camera_frames(self.position, q, *self._views)
+            inv_scale = (1.0 / self.scale).contiguous()
+            loss, depth, no_overlap = 0.0, None, None
+            for v in range(self.depth_obs.shape[0]):
+                p_v, q_v = position_c[v].contiguous(), orientation_c[v].contiguous()
+                loss_depth, depth, _ = render_and_compare(grids, p_v, q_v, inv_scale, self.depth_obs[v],
+                                                          self.threshold, self.camera)
+                loss = loss + self.depth_weight * torch.nan_to_num(loss_depth, nan=0.0)
+                no_overlap = torch.isnan(loss_depth) if no_overlap is None else (no_overlap | torch.isnan(loss_depth))
+                if self.pc_weight and self._view_points[v].shape[0] > 0:
+                    loss = loss + self.pc_weight * losses.point_loss(self._view_points[v], p_v, q_v,
+                                                                     self.scale, grids4)
+            return loss, depth, self.depth_obs[-1], no_overlap  # the last view's inlier ratio (:463)
+        if isinstance(self.decoder, FusedTailDecoder) and self.position.is_cuda \
+                and self.point_counts is None:  # the chained operator takes one shared cloud
+            # decoder tail, render-and-compare and point loss chained through the C ABI (estimation/fused.py):
+            # no dense grid, no separate layout / scaling / add passes
+            dec = self.decoder
+            w, b = dec.tail_parameters()
+            loss, depth, _, loss_depth = decode_render_compare(
+                dec.trunk(self.latent), w, b, self.position, q.contiguous(), self.scale,
+                self.depth_obs, self.points if self.pc_weight and self.points.shape[0] > 0 else None,
+                dec.volume_size, self.threshold, self.camera, base=dec.base,
+                depth_weight=self.depth_weight, pc_weight=self.pc_weight)
+            return loss, depth, self.depth_obs, torch.isnan(loss_depth)
+        grids = self._grids()
+        loss_depth, depth, _ = render_and_compare(grids, self.position, q.contiguous(),
+                                              (1.0 / self.scale).contiguous(), self.depth_obs,
+                                              self.threshold, self.camera)
+        no_overlap = torch.isnan(loss_depth)
+        loss = self.depth_weight * torch.nan_to_num(loss_depth, nan=0.0)
+        if self.pc_weight and self.points.shape[-2] > 0:
+            # NB: the reference passes the un-normalised quaternion and lets pc_loss normalise it
+            # (simple_setup.py:436-443, losses.py:56); q is already unit here, same value
+            loss_pc = losses.point_loss(self.points, self.position, q, self.scale,
+                                        grids if grids.dim() == 4 else grids[None])
+            if self.point_counts is not None:  # mean over the instance's own points, not the padding
+                n = self.point_counts.to(loss_pc.dtype)
+                loss_pc = loss_pc * torch.where(n > 0, self.points.shape[1] / n.clamp(min=1.0),
+                                                torch.zeros_like(n))
+            loss = loss + self.pc_weight * loss_pc
+        return loss, depth, self.depth_obs, no_overlap
 
-        source, target, weight = self.point_constraint
-        return weight * views.point_constraint_loss(self.orientation, source, target)
-
-    def _multiview_step(self) -> torch.Tensor:
-        """One iteration over V views of the same object (simple_setup.py:420-462): the pose is moved
-        into every camera frame, every view is rendered, compared and scored against its own observed
-        points, the losses are summed; autograd carries the gradients back through the rigid maps."""
-        from . import views
-
+    def _torch_step(self) -> torch.Tensor:
         self.optimizer.zero_grad(set_to_none=True)
         q = self.orientation / torch.linalg.norm(self.orientation, dim=1, keepdim=True)
-        grids = self._grids()
-        grids4 = grids if grids.dim() == 4 else grids[None]
-        position_c, orientation_c = views.to_camera_frames(self.position, q, *self._views)
-        inv_scale = (1.0 / self.scale).contiguous()
-        loss, depth, no_overlap = 0.0, None, None
-        for v in range(self.depth_obs.shape[0]):
-            p_v, q_v = position_c[v].contiguous(), orientation_c[v].contiguous()
-            loss_depth, depth, _ = render_and_compare(grids, p_v, q_v, inv_scale, self.depth_obs[v],
-                                                      self.threshold, self.camera)
-            loss = loss + self.depth_weight * torch.nan_to_num(loss_depth, nan=0.0)
-            no_overlap = torch.isnan(loss_depth) if no_overlap is None else (no_overlap | torch.isnan(loss_depth))
-            if self.pc_weight and self._view_points[v].shape[0] > 0:
-                loss = loss + self.pc_weight * losses.point_loss(self._view_points[v], p_v, q_v,
-                                                                 self.scale, grids4)
+        loss, depth, obs, no_overlap = self._torch_loss(q)
         if self.point_constraint is not None:
-            loss = loss + self._constraint_loss()
+            # on the un-normalised orientation (simple_setup.py:164-175)
+            source, target, weight = self.point_constraint
+            loss = loss + weight * views.point_constraint_loss(self.orientation, source, target)
         loss.sum().backward()
         self.optimizer.step()
         with torch.no_grad():
             self.orientation /= torch.linalg.norm(self.orientation, dim=1, keepdim=True)
         if self.inlier_threshold is not None:
-            self._track_best_torch(depth, self.depth_obs[-1])
+            self._track_best_torch(depth, obs)
         self.last_losses = self._reported(loss, no_overlap)
         return self.last_losses
 
@@ -851,67 +841,13 @@ class HypothesisOptimizer:
             return self.last_losses
         return self._eager_step()
 
-    def _fused_loss(self, q: torch.Tensor):
-        """Decoder tail, render-and-compare and point loss chained through the C ABI
-        (estimation/fused.py): no dense grid, no separate layout / scaling / add passes."""
-        dec = self.decoder
-        w, b = dec.tail_parameters()
-        loss, depth, _, loss_depth = decode_render_compare(
-            dec.trunk(self.latent), w, b, self.position, q.contiguous(), self.scale,
-            self.depth_obs, self.points if self.pc_weight and self.points.shape[0] > 0 else None,
-            dec.volume_size, self.threshold, self.camera, base=dec.base,
-            depth_weight=self.depth_weight, pc_weight=self.pc_weight)
-        return loss, depth, torch.isnan(loss_depth)
-
     def _eager_step(self) -> torch.Tensor:
         if self.optimizer_impl == "fused":
             # the C ABI launches on the CURRENT device's stream: make the tensors' device current
             # (OptionalCUDAGuard of sdf_renderer.cpp:58, 82)
             with torch.cuda.device(self.position.device):
                 return self._fused_iteration()
-        if self._views is not None:
-            return self._multiview_step()
-        self.optimizer.zero_grad(set_to_none=True)
-        q = self.orientation / torch.linalg.norm(self.orientation, dim=1, keepdim=True)
-        if isinstance(self.decoder, FusedTailDecoder) and self.position.is_cuda \
-                and self.point_counts is None:  # the chained operator takes one shared cloud
-            loss, depth, no_overlap = self._fused_loss(q)
-            if self.point_constraint is not None:
-                loss = loss + self._constraint_loss()
-            loss.sum().backward()
-            self.optimizer.step()
-            with torch.no_grad():
-                self.orientation /= torch.linalg.norm(self.orientation, dim=1, keepdim=True)
-            if self.inlier_threshold is not None:
-                self._track_best_torch(depth)
-            self.last_losses = self._reported(loss, no_overlap)
-            return self.last_losses
-        grids = self._grids()
-        loss_depth, depth, _ = render_and_compare(grids, self.position, q.contiguous(),
-                                              (1.0 / self.scale).contiguous(), self.depth_obs,
-                                              self.threshold, self.camera)
-        no_overlap = torch.isnan(loss_depth)
-        loss = self.depth_weight * torch.nan_to_num(loss_depth, nan=0.0)
-        if self.pc_weight and self.points.shape[-2] > 0:
-            # NB: the reference passes the un-normalised quaternion and lets pc_loss normalise it
-            # (simple_setup.py:436-443, losses.py:56); q is already unit here, same value
-            loss_pc = losses.point_loss(self.points, self.position, q, self.scale,
-                                        grids if grids.dim() == 4 else grids[None])
-            if self.point_counts is not None:  # mean over the instance's own points, not the padding
-                n = self.point_counts.to(loss_pc.dtype)
-                loss_pc = loss_pc * torch.where(n > 0, self.points.shape[1] / n.clamp(min=1.0),
-                                                torch.zeros_like(n))
-            loss = loss + self.pc_weight * loss_pc
-        if self.point_constraint is not None:
-            loss = loss + self._constraint_loss()
-        loss.sum().backward()
-        self.optimizer.step()
-        with torch.no_grad():
-            self.orientation /= torch.linalg.norm(self.orientation, dim=1, keepdim=True)
-        if self.inlier_threshold is not None:
-            self._track_best_torch(depth)
-        self.last_losses = self._reported(loss, no_overlap)
-        return self.last_losses
+        return self._torch_step()
 
     @staticmethod
     def _reported(loss: torch.Tensor, no_overlap: Optional[torch.Tensor]) -> torch.Tensor:

@@ -125,9 +125,13 @@ def test_reset_reproduces_a_fresh_optimizer(cuda_device):
         assert float((a.position - b.position).abs().max()) < 1e-4
         torch.testing.assert_close(a.best_inlier_ratio, b.best_inlier_ratio, rtol=0, atol=2e-3)
         assert torch.equal(a.best_iteration, b.best_iteration)
+        loaded = [t.clone() for t in (a.depth_obs, a.points, a.position)]
         with pytest.raises(ValueError):
             a.reset(hyp[1]["position"], hyp[1]["orientation"], 1.0 / hyp[1]["inv_scale"],
                     torch.zeros(B, 8, device=dev) if "decoder" in kw else None, torch.full_like(obs[1], 0.7))
+        assert torch.equal(a.depth_obs, obs[1])  # a rejected reset leaves the optimiser untouched
+        for t, want in zip((a.depth_obs, a.points, a.position), loaded):
+            assert torch.equal(t, want)
     with pytest.raises(RuntimeError):
         make(hyp[0], obs[0]).reset(hyp[1]["position"], hyp[1]["orientation"], 1.0 / hyp[1]["inv_scale"],
                                    torch.zeros(B, 8, device=dev), obs[1])  # no capacity: cloud size is baked in
