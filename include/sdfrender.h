@@ -46,7 +46,7 @@
 extern "C" {
 #endif
 
-#define SDFR_ABI_VERSION 10
+#define SDFR_ABI_VERSION 11
 
 #define SDFR_E_NULL (-1)  /* a required pointer is NULL */
 #define SDFR_E_SHAPE (-2) /* resolution < 2, negative sizes, image too large */
@@ -511,6 +511,30 @@ int sdfr_conv3d_forward(const float* x, int batch, int in_channels, int in_size,
 int sdfr_conv3d_backward_data(const float* grad_y, const float* y, int batch, int in_channels,
                               int in_size, const float* weight, int out_channels, int kernel_size,
                               float* grad_x, void* stream);
+
+/*
+ * Observed point clouds of K object instances, without a host synchronisation (the reference builds one
+ * cloud per detection with torch.nonzero: initialization/pointset_utils.py:34-89).
+ * Pixel p of instance k is selected where its masked depth is non-zero:
+ *   masked = depth[k*depth_stride + p], 0 where mask[k*H*W + p] == 0, 0 where masked > far_field
+ * (depth_stride = 0 shares one depth image; mask: bytes 0/1 such as a torch.bool tensor, NULL = no mask;
+ * far_field = +inf for none).  Selected pixels become points in row-major pixel order (the order of
+ * torch.nonzero), in the OpenGL camera frame:
+ *   ((col - cx) * z / fx, -(row - cy) * z / fy, -z),  z = masked depth,
+ * with cx, cy, fx, fy in the pixel-centre-0 convention (Camera.get_pinhole_camera_parameters(0.0)); the
+ * division is a multiplication by the fp32 reciprocal, as torch computes it on CUDA, so the values equal
+ * losses.depth_to_pointcloud's on the same device bit for bit.
+ * Outputs: masked_depth [K,H,W] (NULL skips it); points [K,capacity,3], rows [count, capacity) set to
+ * 1e6 (losses.PAD_COORDINATE: outside every SDF volume); counts [K] int64, the TRUE number of selected
+ * pixels even when it exceeds capacity (only the first `capacity` points are written).  points may be
+ * NULL with capacity 0: counts (and masked_depth) only.  scratch: device memory of the size
+ * sdfr_depth_to_points_scratch reports.  At most 2^30 pixels per image.
+ */
+int sdfr_depth_to_points_scratch(int n_instances, int width, int height, long long* bytes);
+int sdfr_depth_to_points(const float* depth, long long depth_stride, const unsigned char* mask,
+                         int n_instances, int width, int height, float far_field, float fx, float fy,
+                         float cx, float cy, float* masked_depth, float* points, int capacity,
+                         long long* counts, void* scratch, void* stream);
 
 #ifdef __cplusplus
 }

@@ -13,7 +13,7 @@ from ctypes import c_float, c_int, c_longlong, c_uint, c_void_p
 LIB_PATH = os.environ.get("SDFR_LIB_PATH") or os.path.join(
     os.path.dirname(os.path.abspath(__file__)), "libsdfrender.so")
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 GRAD_SDF = 0x01
 GRAD_POSITION = 0x02
@@ -97,6 +97,10 @@ SIGNATURES = {
     "sdfr_upsample3d_backward": (c_int, [_P, c_int, c_int, c_int, _P, _P]),
     "sdfr_conv3d_forward": (c_int, [_P, c_int, c_int, c_int, _P, _P, c_int, c_int, c_int, _P, _P]),
     "sdfr_conv3d_backward_data": (c_int, [_P, _P, c_int, c_int, c_int, _P, c_int, c_int, _P, _P]),
+    "sdfr_depth_to_points_scratch": (c_int, [c_int, c_int, c_int, _P]),
+    "sdfr_depth_to_points": (
+        c_int, [_P, c_longlong, _P, c_int, c_int, c_int, c_float, c_float, c_float, c_float, c_float, _P, _P,
+                c_int, _P, _P, _P]),
     "sdfr_forward_composite": (
         c_int, [_P, c_int, c_longlong, c_int, *_POSE, c_int, *_CAM, c_float, _P, _P, _P, _P]),
     "sdfr_backward_composite": (

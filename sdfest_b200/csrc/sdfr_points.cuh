@@ -232,4 +232,168 @@ int launch_point_loss(PointParams P, int batch, cudaStream_t s) {
   return check_launch("sdfr_point_loss_kernel");
 }
 
+/*
+ * Observed point clouds of K object instances (sdfr_depth_to_points): an ordered compaction of the
+ * selected pixels of every instance, in row-major pixel order (the order of torch.nonzero), so that the
+ * clouds are the ones losses.depth_to_pointcloud builds, bit for bit.
+ *   1. sdfr_points_count_kernel: per (instance, tile of kPtsTile pixels) the number of selected pixels
+ *      (and the masked depth, when asked for);
+ *   2. sdfr_points_scan_kernel: one CTA per instance scans its tile counts into tile offsets (exclusive)
+ *      and writes the instance's true count;
+ *   3. sdfr_points_write_kernel: each tile is selected again, a CTA prefix sum gives every selected
+ *      pixel its row, and rows below the capacity are written; extra CTAs fill rows [count, capacity)
+ *      with the padding coordinate.
+ * Each thread owns kPtsPerThread consecutive pixels, so thread order is pixel order.
+ */
+constexpr int kPtsThreads = 256;
+constexpr int kPtsPerThread = 4;
+constexpr int kPtsTile = kPtsThreads * kPtsPerThread;
+constexpr float kPadCoordinate = 1.0e6f; /* losses.PAD_COORDINATE */
+
+struct ExtractParams {
+  const float* __restrict__ depth;  // [H,W] (depth_stride 0) or [K,H,W]
+  long long depth_stride;
+  const unsigned char* __restrict__ mask;  // [K,H,W] or NULL (= depth != 0)
+  float far_field;
+  float cx, cy, inv_fx, inv_fy;
+  int width, n_pixels, n_tiles, capacity;
+  float* __restrict__ masked_depth;  // [K,H,W] or NULL
+  float* __restrict__ points;        // [K,capacity,3]
+  long long* __restrict__ counts;    // [K]
+  int* __restrict__ tile_offsets;    // [K,n_tiles] scratch: tile counts, then exclusive offsets
+  int z_offset;
+};
+
+/* The masked depth of this thread's pixels (as SDFPipeline._preprocess_depth: 0 outside the mask and
+ * beyond the far field) and a bit per selected pixel (masked depth != 0; NaN is selected, as by
+ * torch.nonzero). */
+__device__ __forceinline__ unsigned select_pixels(const ExtractParams& P, int k, int p0, float v[kPtsPerThread]) {
+  const float* __restrict__ d = P.depth + (size_t)k * P.depth_stride;
+  const unsigned char* __restrict__ m = P.mask ? P.mask + (size_t)k * P.n_pixels : nullptr;
+  unsigned bits = 0;
+#pragma unroll
+  for (int i = 0; i < kPtsPerThread; ++i) {
+    const int p = p0 + i;
+    float x = 0.0f;
+    if (p < P.n_pixels) {
+      x = __ldg(d + p);
+      if (m && !__ldg(m + p)) x = 0.0f;
+      if (x > P.far_field) x = 0.0f;
+    }
+    v[i] = x;
+    if (x != 0.0f) bits |= 1u << i;
+  }
+  return bits;
+}
+
+/* exclusive prefix of `x` over the CTA's threads, and the CTA total */
+__device__ __forceinline__ int cta_exclusive_scan(int x, int* total) {
+  __shared__ int warp_tot[kPtsThreads / 32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int incl = x;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int y = __shfl_up_sync(kFull, incl, o);
+    if (lane >= o) incl += y;
+  }
+  if (lane == 31) warp_tot[warp] = incl;
+  __syncthreads();
+  int before = 0, all = 0;
+#pragma unroll
+  for (int w = 0; w < kPtsThreads / 32; ++w) {
+    const int t = warp_tot[w];
+    before += w < warp ? t : 0;
+    all += t;
+  }
+  __syncthreads(); /* warp_tot may be reused by the caller's next scan */
+  *total = all;
+  return before + incl - x;
+}
+
+__global__ void __launch_bounds__(kPtsThreads) sdfr_points_count_kernel(const __grid_constant__ ExtractParams P) {
+  const int k = blockIdx.y + P.z_offset;
+  const int p0 = blockIdx.x * kPtsTile + threadIdx.x * kPtsPerThread;
+  float v[kPtsPerThread];
+  const unsigned bits = select_pixels(P, k, p0, v);
+  if (P.masked_depth) {
+    float* __restrict__ out = P.masked_depth + (size_t)k * P.n_pixels;
+#pragma unroll
+    for (int i = 0; i < kPtsPerThread; ++i)
+      if (p0 + i < P.n_pixels) out[p0 + i] = v[i];
+  }
+  int total;
+  cta_exclusive_scan(__popc(bits), &total);
+  if (threadIdx.x == 0) P.tile_offsets[(size_t)k * P.n_tiles + blockIdx.x] = total;
+}
+
+/* one CTA per instance: tile counts -> exclusive tile offsets, counts[k] = the instance's total */
+__global__ void __launch_bounds__(kPtsThreads) sdfr_points_scan_kernel(const __grid_constant__ ExtractParams P) {
+  const int k = blockIdx.x;
+  int* __restrict__ t = P.tile_offsets + (size_t)k * P.n_tiles;
+  int carry = 0;
+  for (int i0 = 0; i0 < P.n_tiles; i0 += kPtsThreads) {
+    const int i = i0 + threadIdx.x;
+    const int c = i < P.n_tiles ? t[i] : 0;
+    int total;
+    const int before = cta_exclusive_scan(c, &total);
+    if (i < P.n_tiles) t[i] = carry + before;
+    carry += total;
+  }
+  if (threadIdx.x == 0) P.counts[k] = carry;
+}
+
+__global__ void __launch_bounds__(kPtsThreads) sdfr_points_write_kernel(const __grid_constant__ ExtractParams P) {
+  const int k = blockIdx.y + P.z_offset;
+  float* __restrict__ out = P.points + (size_t)k * P.capacity * 3;
+  if ((int)blockIdx.x >= P.n_tiles) { /* padding rows [count, capacity) */
+    const long long n = P.counts[k];
+    const int r = ((int)blockIdx.x - P.n_tiles) * kPtsThreads + threadIdx.x;
+    if (r < P.capacity && r >= n) {
+      out[3 * (size_t)r + 0] = kPadCoordinate;
+      out[3 * (size_t)r + 1] = kPadCoordinate;
+      out[3 * (size_t)r + 2] = kPadCoordinate;
+    }
+    return;
+  }
+  const int p0 = blockIdx.x * kPtsTile + threadIdx.x * kPtsPerThread;
+  float v[kPtsPerThread];
+  const unsigned bits = select_pixels(P, k, p0, v);
+  int total;
+  int row = P.tile_offsets[(size_t)k * P.n_tiles + blockIdx.x] + cta_exclusive_scan(__popc(bits), &total);
+#pragma unroll
+  for (int i = 0; i < kPtsPerThread; ++i) {
+    if (!(bits & (1u << i))) continue;
+    if (row < P.capacity) {
+      /* losses.depth_to_pointcloud: torch evaluates (col - cx) * z / fx with the division by a Python
+       * scalar as a multiplication by its fp32 reciprocal; explicit roundings keep nvcc from contracting */
+      const int p = p0 + i;
+      const int r = p / P.width, c = p - r * P.width;
+      const float z = v[i];
+      out[3 * (size_t)row + 0] = __fmul_rn(__fmul_rn(__fsub_rn((float)c, P.cx), z), P.inv_fx);
+      out[3 * (size_t)row + 1] = __fmul_rn(__fmul_rn(-__fsub_rn((float)r, P.cy), z), P.inv_fy);
+      out[3 * (size_t)row + 2] = -z;
+    }
+    ++row;
+  }
+}
+
+int launch_depth_to_points(ExtractParams P, int n_instances, cudaStream_t s) {
+  const int n_pad = P.points ? (P.capacity + kPtsThreads - 1) / kPtsThreads : 0;
+  for (int z0 = 0; z0 < n_instances; z0 += 65535) {
+    P.z_offset = z0;
+    const dim3 grid(P.n_tiles, n_instances - z0 < 65535 ? n_instances - z0 : 65535);
+    sdfr_points_count_kernel<<<grid, kPtsThreads, 0, s>>>(P);
+  }
+  P.z_offset = 0;
+  sdfr_points_scan_kernel<<<n_instances, kPtsThreads, 0, s>>>(P);
+  if (P.points) {
+    for (int z0 = 0; z0 < n_instances; z0 += 65535) {
+      P.z_offset = z0;
+      const dim3 grid(P.n_tiles + n_pad, n_instances - z0 < 65535 ? n_instances - z0 : 65535);
+      sdfr_points_write_kernel<<<grid, kPtsThreads, 0, s>>>(P);
+    }
+  }
+  return check_launch("sdfr_depth_to_points");
+}
+
 #endif /* SDFR_POINTS_CUH_ */

@@ -2344,5 +2344,39 @@ int sdfr_conv3d_backward_data(const float* grad_y, const float* y, int batch, in
   return launch_conv3<true>(P, in_channels, batch, (cudaStream_t)stream);
 }
 
+static int points_check(int n_instances, int width, int height) {
+  if (n_instances < 0 || width < 1 || height < 1 || (long long)width * height > (1ll << 30))
+    return fail(SDFR_E_SHAPE, "depth to points: n_instances >= 0 and a non-empty image of at most 2^30 pixels expected");
+  return 0;
+}
+
+int sdfr_depth_to_points_scratch(int n_instances, int width, int height, long long* bytes) {
+  if (int rc = points_check(n_instances, width, height)) return rc;
+  if (!bytes) return fail(SDFR_E_NULL, "depth to points scratch: bytes is NULL");
+  const long long n_tiles = ((long long)width * height + kPtsTile - 1) / kPtsTile;
+  *bytes = (long long)sizeof(int) * n_instances * n_tiles;
+  return 0;
+}
+
+int sdfr_depth_to_points(const float* depth, long long depth_stride, const unsigned char* mask, int n_instances,
+                         int width, int height, float far_field, float fx, float fy, float cx, float cy,
+                         float* masked_depth, float* points, int capacity, long long* counts, void* scratch,
+                         void* stream) {
+  if (int rc = points_check(n_instances, width, height)) return rc;
+  if (depth_stride < 0 || capacity < 0) return fail(SDFR_E_SHAPE, "depth to points: depth_stride >= 0 and capacity >= 0 expected");
+  if (n_instances == 0) return 0;
+  if (!depth || !counts || !scratch) return fail(SDFR_E_NULL, "depth to points: depth, counts or scratch is NULL");
+  if (!points && capacity > 0) return fail(SDFR_E_NULL, "depth to points: points is NULL but capacity > 0");
+  ExtractParams P;
+  memset(&P, 0, sizeof(P));
+  P.depth = depth; P.depth_stride = depth_stride; P.mask = mask; P.far_field = far_field;
+  /* torch's CUDA division of a tensor by a Python scalar multiplies by the reciprocal rounded to fp32 */
+  P.cx = cx; P.cy = cy; P.inv_fx = 1.0f / fx; P.inv_fy = 1.0f / fy;
+  P.width = width; P.n_pixels = width * height; P.n_tiles = (P.n_pixels + kPtsTile - 1) / kPtsTile;
+  P.capacity = capacity; P.masked_depth = masked_depth; P.points = capacity > 0 ? points : nullptr;
+  P.counts = counts; P.tile_offsets = static_cast<int*>(scratch);
+  return launch_depth_to_points(P, n_instances, (cudaStream_t)stream);
+}
+
 #endif
 }  // extern "C"

@@ -107,8 +107,8 @@ class HypothesisOptimizer:
     The reference keeps references to the live tensors there (:207-210), so what it returns is always
     the last iterate (``result("last_iteration")``); the copies are what the code evidently intends.
 
-    Serving many observations with ONE captured graph: ``point_capacity`` (fused path, one shared
-    observation) stores the observed points in a buffer of that fixed size (padding outside every volume,
+    Serving many observations with ONE captured graph: ``point_capacity`` (fused path; a shared observation,
+    views or object instances) stores each observed cloud in a buffer of that fixed size (padding outside every volume,
     where the point loss is exactly 0; the mean is taken over the true count), so that ``reset(...)`` can load
     the next observation and initial estimate into the same device buffers and ``step()`` keeps replaying
     the graph captured for the first one (``SDFPipeline`` does this).
@@ -177,8 +177,8 @@ class HypothesisOptimizer:
                                               capturable=self.position.is_cuda)
         B = self.position.shape[0]
         self.point_capacity, self.max_points = int(point_capacity), int(max_points)
-        if point_capacity and (self.optimizer_impl != "fused" or (not multiview and depth_obs.dim() != 2)):
-            raise ValueError("point_capacity needs the fused path and one shared observation (H,W) or views (V,H,W)")
+        if point_capacity and self.optimizer_impl != "fused":
+            raise ValueError("point_capacity needs the fused path")
         self.last_losses = None
         self.inlier_threshold = None if inlier_threshold is None else float(inlier_threshold)
         if self.inlier_threshold is not None:
@@ -214,10 +214,12 @@ class HypothesisOptimizer:
         they are counted once.  Construction allocates the buffers (private copies: never the caller's tensors);
         reset() overwrites them in place, so a captured graph keeps reading them, and raises before it writes any.
 
-        Object instances (construction only): ``depth_obs`` (K,H,W) and ``instance`` (B,): hypothesis b is compared
-        with the depth map and the points of instance[b] (default: one map per hypothesis)."""
+        Object instances: ``depth_obs`` (K,H,W) and ``instance`` (B,): hypothesis b is compared with the depth map and
+        the points of instance[b] (default: one map per hypothesis); K and the mapping are fixed at construction."""
         B, cap, first = int(self.position.shape[0]), self.point_capacity, self.depth_obs is None
         views = camera_positions is not None or self._views is not None
+        if not first:
+            instance = self.instance
         if first:
             if views:
                 if instance is not None:
@@ -242,19 +244,33 @@ class HypothesisOptimizer:
                 raise RuntimeError(f"depth_obs must have shape (V,{H},{W})" if views
                                    else f"depth_obs must have shape ({H},{W}) or ({B},{H},{W})")
         else:
-            if tuple(depth_obs.shape) != tuple(self.depth_obs.shape):
-                raise ValueError(f"depth_obs must keep its shape {tuple(self.depth_obs.shape)}")
+            shape = tuple(self.depth_obs.shape) if instance is None else (self._n_instances, *self.depth_obs.shape[1:])
+            if tuple(depth_obs.shape) != shape:
+                raise ValueError(f"depth_obs must keep its shape {shape}")
             if self.pc_weight and not cap:
                 raise RuntimeError("a new observation needs point_capacity (the cloud sizes are baked in)")
         if instance is not None:
             clouds, counts = losses.depth_to_pointclouds(depth_obs, self.camera, self.max_points)
-            self.instance = instance
-            self.points = clouds.index_select(0, instance).contiguous()
-            self.point_counts = counts.index_select(0, instance)
-            self.depth_obs = depth_obs.index_select(0, instance).contiguous()
+            if cap and int(counts.max()) > cap:
+                raise ValueError(f"{int(counts.max())} observed points exceed point_capacity {cap}")
             # hypothesis b weighs its own points with pc_weight / counts[b]
-            n = self.point_counts.to(torch.float32)
-            self._up_p = torch.where(n > 0, self.pc_weight / n.clamp(min=1.0), torch.zeros_like(n)).contiguous()
+            n = counts.index_select(0, instance).to(torch.float32)
+            up_p = torch.where(n > 0, self.pc_weight / n.clamp(min=1.0), torch.zeros_like(n))
+            if first:
+                self.instance, self._n_instances = instance, int(depth_obs.shape[0])
+                self.depth_obs = depth_obs.index_select(0, instance).contiguous()
+                self.point_counts = counts.index_select(0, instance)
+                self._up_p = up_p.contiguous()
+                # with point_capacity: fixed-size clouds, padded outside every volume (point loss exactly 0 there)
+                self.points = clouds.index_select(0, instance).contiguous() if not cap else \
+                    torch.empty((B, cap, 3), dtype=torch.float32, device=clouds.device)
+            else:
+                self.depth_obs.copy_(depth_obs.index_select(0, instance))
+                self.point_counts.copy_(counts.index_select(0, instance))
+                self._up_p.copy_(up_p)
+            if cap:
+                self.points.fill_(losses.PAD_COORDINATE)
+                self.points[:, :clouds.shape[1]].copy_(clouds.index_select(0, instance))
         else:
             V = int(depth_obs.shape[0]) if views else 1
             poses = [None if p is None else p.detach().reshape(V, k)
@@ -303,13 +319,12 @@ class HypothesisOptimizer:
         """Start over from a new initial estimate -- and, with ``depth_obs``, a new observation -- in the SAME
         device buffers: optimiser state, result selection and losses are cleared, and a captured graph stays
         valid (``step()`` keeps replaying it).  Fused path only; a new observation needs ``point_capacity``
-        (or ``pc_weight`` 0).  With views: ``depth_obs`` (V,H,W) and, optionally, new camera poses.  The point
+        (or ``pc_weight`` 0).  With views: ``depth_obs`` (V,H,W) and, optionally, new camera poses.  With object
+        instances: ``depth_obs`` (K,H,W), the same K and ``instance`` mapping as at construction.  The point
         constraint, if any, stays the one given at construction.  Raises ValueError when a new cloud does not
         fit the capacity."""
         if self.optimizer_impl != "fused":
             raise RuntimeError("reset() is for optimizer='fused'")
-        if self.point_counts is not None:
-            raise RuntimeError("reset() supports one shared observation or views (no object instances)")
         if not self._V and (camera_positions is not None or camera_orientations is not None):
             raise ValueError("camera poses can only be reset on an optimiser constructed with views")
         if self.latent is not None and latent is None:

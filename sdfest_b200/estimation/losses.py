@@ -7,20 +7,102 @@ for them as the next step after the renderer).
 """
 from __future__ import annotations
 
+import ctypes
+from typing import Optional
+
 import torch
 
 
 def depth_to_pointcloud(depth_image: torch.Tensor, camera, mask=None) -> torch.Tensor:
     """Observed depth (H,W) -> points (N,3) in the OpenGL camera frame (x right, y up, z back).
 
-    Uses the pixel-centre-0 principal point like the reference (pointset_utils.py:57).  The
-    nonzero() makes this a host sync; it runs once per observation, outside the loop.
+    Uses the pixel-centre-0 principal point like the reference (pointset_utils.py:57).  Reading the
+    number of points is a host sync; it runs once per observation, outside the loop.  fp32 CUDA tensors go
+    through ``sdfr_depth_to_points`` (same points, same order, same bits as the torch expression on CUDA).
     """
+    if depth_image.is_cuda and depth_image.dtype == torch.float32 and depth_image.dim() == 2:
+        sel = None if mask is None else (depth_image * mask) != 0  # the torch expression's selection
+        _, points, _ = extract_instances(depth_image[None], None if sel is None else sel[None], camera)
+        return points[0]
     fx, fy, cx, cy, _ = camera.get_pinhole_camera_parameters(0.0)
     img = depth_image if mask is None else depth_image * mask
     rows, cols = torch.nonzero(img, as_tuple=True)
     z = depth_image[rows, cols]
     return torch.stack([(cols.float() - cx) * z / fx, -(rows.float() - cy) * z / fy, -z], dim=1)
+
+
+def extract_instances(depth: torch.Tensor, masks: Optional[torch.Tensor], camera, far_field: Optional[float] = None,
+                      capacity: int = 0):
+    """The observations of K object instances in one pass of ``sdfr_depth_to_points``:
+    ``(masked_depth (K,H,W), points (K,M,3), counts (K,) int64)``.
+
+    ``depth`` (H,W) is shared by all instances, or (K,H,W) is one map each; ``masks`` (K,H,W) bool or None
+    (every non-zero pixel).  The masked depth is 0 outside the mask and beyond ``far_field``, as
+    ``SDFPipeline`` preprocesses a view; the caller's ``depth`` is not modified.  Row k of ``points`` holds
+    instance k's cloud (``depth_to_pointcloud`` of its masked depth, bit for bit) followed by
+    ``PAD_COORDINATE`` rows.  M = ``capacity``, or the largest count when ``capacity`` is 0; ``counts`` are
+    the true counts even where they exceed ``capacity`` (only the first ``capacity`` points are kept).
+    On CUDA (fp32) this is ``sdfr_depth_to_points``: with ``capacity`` > 0 nothing synchronises with the host;
+    with 0, reading the largest count does, once.  CPU tensors take the torch statement of the same."""
+    from .. import _lib
+    from ..differentiable_renderer.sdf_renderer import _on_device_of, _stream
+
+    if depth.is_cuda and depth.dtype != torch.float32:
+        raise RuntimeError("extract_instances takes a float32 depth on CUDA")
+    if depth.dim() not in (2, 3):
+        raise ValueError(f"depth must be (H,W) or (K,H,W), got {tuple(depth.shape)}")
+    H, W = int(depth.shape[-2]), int(depth.shape[-1])
+    if masks is not None:
+        if masks.dtype != torch.bool or masks.dim() != 3 or tuple(masks.shape[1:]) != (H, W) \
+                or masks.device != depth.device:
+            raise ValueError(f"masks must be a bool (K,{H},{W}) tensor on {depth.device}")
+        masks = masks.contiguous()
+    if depth.dim() == 2 and masks is None:
+        raise ValueError("a shared depth image (H,W) needs masks (K,H,W)")
+    K = int(masks.shape[0]) if masks is not None else int(depth.shape[0])
+    if depth.dim() == 3 and int(depth.shape[0]) != K:
+        raise ValueError(f"depth has {int(depth.shape[0])} maps for {K} masks")
+    if capacity < 0:
+        raise ValueError("capacity must be >= 0")
+    depth = depth.contiguous()
+    stride = 0 if depth.dim() == 2 else H * W
+    far = float("inf") if far_field is None else float(far_field)
+    if not depth.is_cuda:
+        masked = depth if masks is None else torch.where(masks, depth, torch.zeros_like(depth))
+        masked = torch.where(masked > far, torch.zeros_like(masked), masked)
+        clouds = [depth_to_pointcloud(d, camera) for d in masked]
+        counts = torch.tensor([int(c.shape[0]) for c in clouds], dtype=torch.int64)
+        M = capacity or max([int(c.shape[0]) for c in clouds], default=0)
+        points = torch.full((K, M, 3), PAD_COORDINATE, dtype=torch.float32)
+        for k, c in enumerate(clouds):
+            points[k, :min(int(c.shape[0]), M)] = c[:M]
+        return masked.contiguous(), points, counts
+    fx, fy, cx, cy, _ = camera.get_pinhole_camera_parameters(0.0)
+    lib = _lib.lib()
+    with _on_device_of(depth):
+        dev = depth.device
+        masked = torch.empty((K, H, W), dtype=torch.float32, device=dev)
+        counts = torch.empty((K,), dtype=torch.int64, device=dev)
+        n = ctypes.c_longlong(0)
+        _lib.check(lib.sdfr_depth_to_points_scratch(K, W, H, ctypes.byref(n)), "sdfr_depth_to_points_scratch")
+        scratch = torch.empty((max(n.value, 1),), dtype=torch.uint8, device=dev)
+
+        def run(masked_out, points, cap):
+            _lib.check(lib.sdfr_depth_to_points(
+                depth.data_ptr(), stride, None if masks is None else masks.data_ptr(), K, W, H, far, fx, fy, cx, cy,
+                None if masked_out is None else masked_out.data_ptr(), None if points is None else points.data_ptr(),
+                cap, counts.data_ptr(), scratch.data_ptr(), _stream()), "sdfr_depth_to_points")
+
+        if capacity:
+            points = torch.empty((K, capacity, 3), dtype=torch.float32, device=dev)
+            run(masked, points, capacity)
+        else:
+            run(masked, None, 0)  # the counts first: they size the clouds
+            M = int(counts.max()) if K else 0
+            points = torch.empty((K, M, 3), dtype=torch.float32, device=dev)
+            if M:
+                run(None, points, M)
+    return masked, points, counts
 
 
 def subsample_points(points: torch.Tensor, max_points: int) -> torch.Tensor:
@@ -41,12 +123,24 @@ def depth_to_pointclouds(depth_images: torch.Tensor, camera, max_points: int = 0
     Instance k owns the first counts[k] points of row k (``depth_to_pointcloud`` + ``subsample_points``
     of its own map); the rest of the row is padding far outside any SDF volume, where the reference's
     ``pc_loss`` is exactly 0 (estimation/losses.py:84-101), so a mean over the instance's own points is
-    ``sum / counts[k]``.  M = the largest count (at least 1).  One host sync per instance, once per
-    observation, outside the loop.
+    ``sum / counts[k]``.  M = the largest count (at least 1).  Once per observation, outside the loop: fp32
+    CUDA tensors take one ``extract_instances`` call (one host sync, a second with ``max_points`` for the
+    per-instance sub-sampling), others one host sync per instance.
     """
     if depth_images.dim() != 3:
         raise RuntimeError(f"depth_images must be (K,H,W), got {tuple(depth_images.shape)}")
-    clouds = [subsample_points(depth_to_pointcloud(d, camera), max_points) for d in depth_images]
+    if depth_images.is_cuda and depth_images.dtype == torch.float32:
+        _, points, counts = extract_instances(depth_images, None, camera)
+        if max_points and points.shape[1] > max_points:
+            clouds = [points[k, :n] for k, n in enumerate(counts.tolist())]
+        elif points.shape[1] == 0:
+            return torch.full((points.shape[0], 1, 3), PAD_COORDINATE, dtype=torch.float32,
+                              device=depth_images.device), counts
+        else:
+            return points, counts
+    else:
+        clouds = [depth_to_pointcloud(d, camera) for d in depth_images]
+    clouds = [subsample_points(c, max_points) for c in clouds]
     counts = torch.tensor([c.shape[0] for c in clouds], dtype=torch.int64)
     M = max(int(counts.max()) if len(clouds) else 0, 1)
     out = torch.full((len(clouds), M, 3), PAD_COORDINATE, dtype=torch.float32, device=depth_images.device)

@@ -16,6 +16,8 @@ constraint ``sdfr_point_constraint``), replayed from a CUDA graph.  A decoder th
 interpolate-to-volume + 1x1x1 convolution runs through ``vae.decode`` and the autograd-composed
 operators.  ``n_hypotheses`` > 1 (an extension) perturbs the initial pose and returns the best
 hypothesis: highest best inlier ratio under ``best_inlier_ratio``, else lowest final loss.
+``estimate_instances`` (an extension) runs that loop for every detection of a frame at once: the reference
+runs ``__call__`` once per detection (estimation/scripts/real_data.py).
 """
 from __future__ import annotations
 
@@ -50,7 +52,8 @@ class SDFPipeline:
     ``profile`` (False): record ``last_timings``.
     ``vae``: a module with ``decode(latent) -> (B,1,R,R,R)`` and a ``decoder`` attribute (the reference's
     ``SDFVAE``); ``init_network``: ``points (1,M,3) | depth (1,H,W) -> (latent, position, scale,
-    orientation representation)`` (the reference's ``SDFPoseNet``).
+    orientation representation)`` (the reference's ``SDFPoseNet``), batched over rows for
+    ``estimate_instances`` (every detection of a frame in one call).
     """
 
     def __init__(self, config: dict, vae: torch.nn.Module, init_network: torch.nn.Module):
@@ -159,16 +162,7 @@ class SDFPipeline:
             if camera_orientations is not None:
                 camera_orientations = camera_orientations.unsqueeze(0)
         n_imgs, dev = depth_images.shape[0], depth_images.device
-        marks = []
-
-        def mark(name):
-            if self.config.get("profile", False):
-                import time
-
-                if depth_images.is_cuda:
-                    torch.cuda.synchronize(dev)
-                marks.append((name, time.perf_counter()))
-
+        marks, mark = self._phase_marks(dev)
         mark("start")
         world_is_camera = camera_positions is None and camera_orientations is None and n_imgs == 1
         if camera_positions is None:
@@ -190,6 +184,148 @@ class SDFPipeline:
                 orientation.repeat(n_hyp, 1) + 0.1 * noise(n_hyp, 4) * (torch.arange(n_hyp, device=dev) > 0)[:, None], dim=1)
             scale, latent = scale.repeat(n_hyp), latent.repeat(n_hyp, 1)
 
+        if world_is_camera:
+            obs, extra = depth_images[0].contiguous(), {}
+        else:
+            obs = depth_images.contiguous()
+            extra = dict(camera_positions=camera_positions, camera_orientations=camera_orientations)
+        # the view loop bakes in the number of views
+        opt = self._optimize(obs, position, orientation, scale, latent, shape_optimization, n_hyp,
+                             0 if world_is_camera else n_imgs, None, point_constraint, mark, **extra)
+        position, orientation, scale, latent_out = opt.result(self.result_selection_strategy)
+        if latent_out is None:
+            latent_out = latent
+        if n_hyp > 1:
+            if self.result_selection_strategy == "best_inlier_ratio":
+                best = int(torch.argmax(torch.nan_to_num(opt.best_inlier_ratio, nan=-1.0)))
+            else:
+                best = int(torch.argmin(torch.nan_to_num(opt.last_losses, nan=float("inf"))))
+            position, orientation = position[best:best + 1], orientation[best:best + 1]
+            scale, latent_out = scale[best:best + 1], latent_out[best:best + 1]
+        # the optimiser's buffers are reused by the next call (`reuse_graph`): hand out copies
+        position, orientation, scale, latent_out = (t.detach().clone() for t in (position, orientation, scale, latent_out))
+        mark("result")
+        if marks:
+            self.last_timings = {b[0] + "_ms": (b[1] - a[1]) * 1e3 for a, b in zip(marks[:-1], marks[1:])}
+        return position, orientation, scale, latent_out
+
+    def estimate_instances(self, depth_image: torch.Tensor, masks: torch.Tensor,
+                           color_image: Optional[torch.Tensor] = None, shape_optimization: bool = True) -> tuple:
+        """Pose, size and latent shape of every detection of one frame in one call: ``depth_image`` (H,W) and
+        ``masks`` (K,H,W) bool, one per detection; one view, in the camera frame.  Returns (position (K,3),
+        orientation (K,4), scale (K,), latent (K,L)); row k is what ``__call__(depth_image, masks[k])`` returns.
+
+        Unlike ``__call__``, the caller's depth image is NOT modified: the K masked depths (mask and far field
+        applied, as ``__call__`` does in place) and their clouds come from one ``extract_instances`` call.
+        Raises ``NoDepthError`` naming the detections without any depth after masking, before any network runs.
+        The initialisation network runs once on all K detections; the loop optimises K x ``n_hypotheses``
+        hypotheses together, each against its own detection, and keeps per detection the hypothesis
+        ``result_selection_strategy`` ranks best.  With ``reuse_graph`` a later frame with as many detections
+        replays the captured iteration of the first.
+        """
+        if depth_image.dim() != 2 or masks.dim() != 3 or tuple(masks.shape[1:]) != tuple(depth_image.shape):
+            raise ValueError("depth_image (H,W) and masks (K,H,W) expected")
+        K, dev = int(masks.shape[0]), depth_image.device
+        marks, mark = self._phase_marks(dev)
+        mark("start")
+        with torch.no_grad():
+            masked, points, counts = losses.extract_instances(depth_image, masks.to(torch.bool), self.cam,
+                                                              self._far_field)
+            n_points = counts.tolist()
+            empty = [k for k, n in enumerate(n_points) if n == 0]
+            if empty:
+                raise NoDepthError(f"no valid depth after masking for detections {empty}")
+            latent, position, scale, orientation = self._nn_init_instances(masked, points, counts)
+        mark("preprocess_and_init_network")
+        n_hyp = int(self.config.get("n_hypotheses", 1))
+        if n_hyp > 1:  # every detection gets the perturbation rows __call__ uses, hypothesis 0 unperturbed
+            g = torch.Generator(device="cpu").manual_seed(0)
+            noise = lambda *s: torch.randn(*s, generator=g).to(dev)  # noqa: E731
+            d_position = 0.02 * noise(n_hyp, 3) * (torch.arange(n_hyp, device=dev) > 0)[:, None]
+            d_orientation = 0.1 * noise(n_hyp, 4) * (torch.arange(n_hyp, device=dev) > 0)[:, None]
+            position = position.repeat_interleave(n_hyp, 0) + d_position.repeat(K, 1)
+            orientation = torch.nn.functional.normalize(
+                orientation.repeat_interleave(n_hyp, 0) + d_orientation.repeat(K, 1), dim=1)
+            scale, latent = scale.repeat_interleave(n_hyp), latent.repeat_interleave(n_hyp, 0)
+        instance = torch.arange(K, device=dev).repeat_interleave(n_hyp)
+        opt = self._optimize(masked, position, orientation, scale, latent, shape_optimization, n_hyp,
+                             ("instances", K), max(n_points), None, mark, instance=instance)
+        position, orientation, scale, latent_out = opt.result(self.result_selection_strategy)
+        if latent_out is None:
+            latent_out = latent
+        if n_hyp > 1:
+            if self.result_selection_strategy == "best_inlier_ratio":
+                best = torch.argmax(torch.nan_to_num(opt.best_inlier_ratio, nan=-1.0).view(K, n_hyp), dim=1)
+            else:
+                best = torch.argmin(torch.nan_to_num(opt.last_losses, nan=float("inf")).view(K, n_hyp), dim=1)
+            rows = torch.arange(K, device=best.device) * n_hyp + best
+            position, orientation, scale, latent_out = (t.index_select(0, rows.to(t.device))
+                                                        for t in (position, orientation, scale, latent_out))
+        # the optimiser's buffers are reused by the next call (`reuse_graph`): hand out copies
+        position, orientation, scale, latent_out = (t.detach().clone() for t in (position, orientation, scale, latent_out))
+        mark("result")
+        if marks:
+            self.last_timings = {b[0] + "_ms": (b[1] - a[1]) * 1e3 for a, b in zip(marks[:-1], marks[1:])}
+        return position, orientation, scale, latent_out
+
+    def _nn_init_instances(self, masked, points, counts) -> Tuple:
+        """Initial (latent (K,L), position (K,3), scale (K,), orientation (K,4)) in the camera frame from ONE call
+        of the initialisation network on all K detections (``_nn_init`` row by row).  A point-set backbone gets
+        every cloud centred on its own centroid and padded to the largest one by repeating its own points
+        cyclically: a max-pooled point network gives what it gives on the unpadded cloud."""
+        head = self.init_config.get("head", {})
+        repr_ = head.get("orientation_repr", "quaternion")
+        if self.config.get("init_view", "first") != "first":
+            raise NotImplementedError('Only the "first" init strategy is supported ("best" ranks the '
+                                      "views by their SO3-grid posterior)")
+        centroid = None
+        if self.init_config.get("backbone_type", "VanillaPointNet") == "VanillaPointNet":
+            K, M = int(points.shape[0]), int(points.shape[1])
+            rows = torch.arange(M, device=points.device)
+            own = (rows[None, :] % counts[:, None])[..., None].expand(K, M, 3)
+            inp = torch.gather(points, 1, own)
+            if self.init_config.get("normalize_pose", True):
+                valid = (rows[None, :] < counts[:, None])[..., None]
+                centroid = torch.where(valid, points, 0.0).sum(1) / counts[:, None].to(points.dtype)
+                inp = inp - centroid[:, None]
+        else:
+            inp = masked
+        latent, position, scale, orientation_repr = self.init_network(inp)
+        latent, position, scale = latent.clone(), position.clone(), scale.clone()
+        if self.config.get("mean_shape", False):
+            latent = torch.zeros_like(latent)
+        if centroid is not None:
+            position = position + centroid
+        if repr_ == "quaternion":
+            orientation = orientation_repr
+        elif repr_ == "discretized":  # the network's own SO3 grid, the argmax of every row
+            index = torch.softmax(orientation_repr, -1).argmax(-1).tolist()
+            orientation = torch.tensor([self.init_network._head._grid.index_to_quat(i) for i in index],
+                                       dtype=torch.float, device=position.device).reshape(-1, 4)
+        else:
+            raise NotImplementedError("Orientation representation is not supported")
+        return latent, position, scale.reshape(-1), orientation
+
+    def _phase_marks(self, dev):
+        """(marks, mark): ``mark(name)`` records the wall time of a phase boundary when ``profile`` is on."""
+        marks = []
+
+        def mark(name):
+            if self.config.get("profile", False):
+                import time
+
+                if dev.type == "cuda":
+                    torch.cuda.synchronize(dev)
+                marks.append((name, time.perf_counter()))
+
+        return marks, mark
+
+    def _optimize(self, obs, position, orientation, scale, latent, shape_optimization, n_hyp, shape_key, n_obs,
+                  point_constraint, mark, **extra) -> HypothesisOptimizer:
+        """The loop of one call from the initial estimate: a HypothesisOptimizer on ``obs`` (``extra``: camera poses
+        or object instances), captured and replayed, or -- ``reuse_graph`` -- the captured one of an earlier call
+        of the same shape, reset to this call's observation.  ``shape_key``: what else the captured iteration bakes
+        in (number of views, number of instances); ``n_obs``: the largest observed cloud when the caller knows it."""
         kw = dict(depth_weight=self.config.get("depth_weight", 1.0), pc_weight=self.config.get("pc_weight", 3.0),
                   max_points=int(self.config.get("max_points", 0)),
                   inlier_threshold=self._relative_inlier_threshold, point_constraint=point_constraint)
@@ -198,11 +334,8 @@ class SDFPipeline:
         else:
             with torch.no_grad():
                 kw.update(sdf=self.vae.decode(latent)[:, 0].contiguous())
-        if world_is_camera:
-            obs = depth_images[0].contiguous()
-        else:
-            obs = depth_images.contiguous()
-            kw.update(camera_positions=camera_positions, camera_orientations=camera_orientations)
+        kw.update(extra)
+        dev = obs.device
         n_it = int(self.config.get("max_iterations", 50))
         use_graph = self.config.get("cuda_graph", True) and n_it > 8
         # one captured iteration serves every call of the same shape (see `reuse_graph` above)
@@ -216,21 +349,22 @@ class SDFPipeline:
                    float(kw["depth_weight"]), float(kw["pc_weight"]), int(kw["max_points"]),
                    float(kw["inlier_threshold"]), self.cam.width, self.cam.height, self.cam.fx, self.cam.fy,
                    self.cam.cx, self.cam.cy, self.cam.pixel_center, get_sdf_grad_mode(), get_empty_space_policy(),
-                   # the view loop bakes in the number of views; the point constraint's source / target / weight
+                   # shape_key: what the loop bakes in besides; the point constraint's source / target / weight
                    # are launch arguments (host values) of the captured sdfr_point_constraint
-                   0 if world_is_camera else n_imgs,
+                   shape_key,
                    None if point_constraint is None else tuple(
                        (float(v) for v in torch.as_tensor(point_constraint[0]).flatten().tolist()
                         + torch.as_tensor(point_constraint[1]).flatten().tolist() + [float(point_constraint[2])])))
-            # the largest cloud of the call (one per view) decides whether the cached buffers fit
-            n_obs = int((obs != 0).flatten(-2).sum(-1).max()) if kw["pc_weight"] else 0
+            # the largest cloud of the call (one per view or instance) decides whether the cached buffers fit
+            if not kw["pc_weight"]:
+                n_obs = 0
+            elif n_obs is None:
+                n_obs = int((obs != 0).flatten(-2).sum(-1).max())
             n_pts = min(n_obs, kw["max_points"]) if kw["max_points"] else n_obs
             cached = self._graph_cache.get(key)
             if cached is not None and n_pts <= cached.point_capacity <= 2 * n_pts + 8192:
-                if world_is_camera:
-                    cached.reset(position, orientation, scale, latent, obs)
-                else:
-                    cached.reset(position, orientation, scale, latent, obs, camera_positions, camera_orientations)
+                cached.reset(position, orientation, scale, latent, obs, extra.get("camera_positions"),
+                             extra.get("camera_orientations"))
                 opt, done = cached, -1  # every iteration of this call is a replay
             else:
                 kw["point_capacity"] = max(4096, -(-n_pts // 4096) * 4096 + 4096)  # room for the next clouds
@@ -248,19 +382,4 @@ class SDFPipeline:
         for _ in range(n_it - done):
             opt.step()
         mark("iterations")
-        position, orientation, scale, latent_out = opt.result(self.result_selection_strategy)
-        if latent_out is None:
-            latent_out = latent
-        if n_hyp > 1:
-            if self.result_selection_strategy == "best_inlier_ratio":
-                best = int(torch.argmax(torch.nan_to_num(opt.best_inlier_ratio, nan=-1.0)))
-            else:
-                best = int(torch.argmin(torch.nan_to_num(opt.last_losses, nan=float("inf"))))
-            position, orientation = position[best:best + 1], orientation[best:best + 1]
-            scale, latent_out = scale[best:best + 1], latent_out[best:best + 1]
-        # the optimiser's buffers are reused by the next call (`reuse_graph`): hand out copies
-        position, orientation, scale, latent_out = (t.detach().clone() for t in (position, orientation, scale, latent_out))
-        mark("result")
-        if marks:
-            self.last_timings = {b[0] + "_ms": (b[1] - a[1]) * 1e3 for a, b in zip(marks[:-1], marks[1:])}
-        return position, orientation, scale, latent_out
+        return opt
