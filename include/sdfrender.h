@@ -46,7 +46,7 @@
 extern "C" {
 #endif
 
-#define SDFR_ABI_VERSION 11
+#define SDFR_ABI_VERSION 12
 
 #define SDFR_E_NULL (-1)  /* a required pointer is NULL */
 #define SDFR_E_SHAPE (-2) /* resolution < 2, negative sizes, image too large */
@@ -55,10 +55,6 @@ extern "C" {
 /* sdf_layout */
 #define SDFR_LAYOUT_DENSE 0
 #define SDFR_LAYOUT_SKEWED 1
-/* EXPERIMENTAL (the A/B of DESIGN.md section 5, not used by the product paths): a float2 per voxel,
- * (v[z], v[z+1]), made by sdfr_zpair_grids; resolution 64 only, accepted by sdfr_compare_forward and
- * sdfr_compare_fused only */
-#define SDFR_LAYOUT_ZPAIR 2
 
 /* flags of the backward entry points */
 #define SDFR_GRAD_SDF 0x01u
@@ -103,11 +99,6 @@ int sdfr_skewed_pitches(int resolution, int* pitch_y, int* pitch_x, long long* e
  */
 int sdfr_skew_grids(const float* sdf, int resolution, long long sdf_stride, int batch,
                     float* skewed, long long skewed_stride, void* stream);
-
-/* EXPERIMENTAL z-pair layout: floats one z-pair grid occupies; dense grids -> z-pair copies (one pass). */
-int sdfr_zpair_elems(int resolution, long long* elems);
-int sdfr_zpair_grids(const float* sdf, int resolution, long long sdf_stride, int batch, float* zpair,
-                     long long zpair_stride, void* stream);
 
 /*
  * Cell bounds of a grid: the first / last CELL index per axis (cell i spans voxels i and i+1) whose

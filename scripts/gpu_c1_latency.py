@@ -1,6 +1,6 @@
 """C1 (ONE 640x480 / 64^3 frame) as a latency problem: where the ~20 us of a single forward launch go.
 
-  * the launch as shipped, as a function of the number of CTAs (SDFR_TARGET_CTAS);
+  * the launch as shipped;
   * crops of the same frame rendered with a shifted principal point (identical rays): one 32x8 tile that
     holds the frame's longest sphere trace (43 samples; found with the CPU oracle, see DESIGN.md), one
     tile of box pixels that miss the surface after a few samples, one tile outside the box -- i.e. launch +
@@ -103,13 +103,6 @@ for name, (tx, ty) in {"tile_longest_trace": (11, 37), "tile_box_miss": (5, 30),
 # the rows of tiles through the object, 640 x 8 and 640 x 64
 out["crop_rows_8"] = timed(lambda: fwd(640, 8, 0, 8 * 37))
 out["crop_rows_64"] = timed(lambda: fwd(640, 64, 0, 8 * 30))
-sweep = {}
-for target in (148, 296, 444, 592, 740, 1200):
-    os.environ["SDFR_TARGET_CTAS"] = str(target)
-    fwd()
-    sweep[target] = {"fwd": timed(fwd), "bwd": timed(bwd), "fused": timed(fused)}
-os.environ.pop("SDFR_TARGET_CTAS")
-out["cta_sweep"] = sweep
 tag = sys.argv[1] if len(sys.argv) > 1 else "c1"
 os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
 with open(os.path.join(ROOT, "gpurun_out", f"{tag}_c1_latency.json"), "w") as f:

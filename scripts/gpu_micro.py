@@ -1,6 +1,6 @@
 """GPU micro-measurements that guide kernel work (not a bench line):
   1. C1: one 640x480 / 64^3 frame forward+backward, ours vs the reference CUDA extension;
-  2. C2 kernels (64 hypotheses) as a function of the number of persistent CTAs (SDFR_TARGET_CTAS).
+  2. C2 kernels (64 hypotheses) in the dense and skewed layouts.
 Writes JSON to gpurun_out/<tag>_micro.json."""
 import json
 import os
@@ -173,13 +173,6 @@ out["c2_layouts"] = {
     "bwd_skewed_sdf_only": timed(lambda: bwd(1, 0x01 | _lib.ZERO_GRADS)),
     "bwd_skewed_no_memset": timed(lambda: bwd(1, _lib.GRAD_ALL)),
 }
-sweep = {}
-for target in (1184, 2368, 4736, 9472):
-    os.environ["SDFR_TARGET_CTAS"] = str(target)
-    fwd()
-    sweep[target] = {"fwd": timed(fwd), "fused": timed(fused), "bwd": timed(bwd)}
-os.environ.pop("SDFR_TARGET_CTAS")
-out["c2_cta_sweep"] = sweep
 tag = sys.argv[1] if len(sys.argv) > 1 else "micro"
 os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
 with open(os.path.join(ROOT, "gpurun_out", f"{tag}_micro.json"), "w") as f:

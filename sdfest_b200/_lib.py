@@ -9,11 +9,12 @@ import ctypes
 import os
 from ctypes import c_float, c_int, c_longlong, c_uint, c_void_p
 
-# SDFR_LIB_PATH: tuning experiments load an alternative build of the SAME library (scripts/)
+# SDFR_LIB_PATH: load another build of the same ABI instead, e.g. a parent commit's, to compare
+# two builds in one process (scripts/ab/)
 LIB_PATH = os.environ.get("SDFR_LIB_PATH") or os.path.join(
     os.path.dirname(os.path.abspath(__file__)), "libsdfrender.so")
 
-ABI_VERSION = 11
+ABI_VERSION = 12
 
 GRAD_SDF = 0x01
 GRAD_POSITION = 0x02
@@ -28,7 +29,6 @@ STEP_NO_UPDATE = 0x200
 TRACK_KEEP_VALID = 0x400  # sdfr_track_best: CLEAR_INPUTS zeroes n_inlier only
 LAYOUT_DENSE = 0
 LAYOUT_SKEWED = 1
-LAYOUT_ZPAIR = 2  # experimental (A/B only)
 
 _P = c_void_p
 _CAM = [c_int, c_int, c_float, c_float, c_float, c_float]  # W, H, cx, cy, fx, fy
@@ -63,8 +63,6 @@ SIGNATURES = {
         c_int, [_P, c_int, c_longlong, c_int, *_POSE, c_int, *_CAM, c_float, _P, c_longlong, _P, _P, _P,
                 c_float, _P, *_GRADS, c_uint, _P, _P]),
     "sdfr_skewed_pitches": (c_int, [c_int, _P, _P, _P]),
-    "sdfr_zpair_elems": (c_int, [c_int, _P]),
-    "sdfr_zpair_grids": (c_int, [_P, c_int, c_longlong, c_int, _P, c_longlong, _P]),
     "sdfr_skew_grids": (c_int, [_P, c_int, c_longlong, c_int, _P, c_longlong, _P]),
     "sdfr_scale_grads": (c_int, [_P, _P, c_int, c_int, *_GRADS, c_uint, _P, c_longlong, _P]),
     "sdfr_point_loss_forward": (

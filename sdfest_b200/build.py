@@ -51,15 +51,12 @@ def up_to_date() -> bool:
 def build(force: bool = False, verbose: bool = False) -> str:
     if not force and up_to_date():
         return LIB_PATH
-    extra = os.environ.get("SDFR_NVCC_EXTRA", "").split()  # tuning experiments (-DSDFR_FWD_BLOCKS=4)
     nvcc = find_nvcc()
-    out_lib = os.environ.get("SDFR_BUILD_OUT") or LIB_PATH  # tuning experiments build a second library
     os.makedirs(OBJ_DIR, exist_ok=True)
-    tag = "".join(c if c.isalnum() else "_" for c in os.path.basename(out_lib))
     objs, procs = [], []
     for part in range(1, N_PARTS + 1):
-        obj = os.path.join(OBJ_DIR, f"{tag}_part{part}.o")
-        cmd = [nvcc, *NVCC_FLAGS, *extra, f"-DSDFR_PART={part}", "-c", *SOURCES, "-o", obj]
+        obj = os.path.join(OBJ_DIR, f"sdfrender_part{part}.o")
+        cmd = [nvcc, *NVCC_FLAGS, f"-DSDFR_PART={part}", "-c", *SOURCES, "-o", obj]
         if verbose:
             cmd[1:1] = ["-Xptxas", "-v"]
             print(" ".join(cmd))
@@ -77,8 +74,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
             failed = subprocess.CalledProcessError(rc, cmd)
     if failed is not None:
         raise failed
-    subprocess.check_call([nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", *objs, "-o", out_lib])
-    return out_lib
+    subprocess.check_call([nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", *objs, "-o", LIB_PATH])
+    return LIB_PATH
 
 
 if __name__ == "__main__":

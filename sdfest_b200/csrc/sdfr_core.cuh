@@ -34,12 +34,8 @@
 #define SDFR_SUB(a, b) __fsub_rn((a), (b))
 /* slab quotients: MUFU.RCP + FMUL (2 ulp) instead of the IEEE division sequence (~9 instructions and
  * a slow-path branch, six times per pixel = 7 % of the fused kernel's instructions); |f| <= 1 here, far
- * from __fdividef's 2^126 caveat.  -DSDFR_EXACT_SLAB_DIV restores the correctly rounded quotient. */
-#ifdef SDFR_EXACT_SLAB_DIV
-#define SDFR_SLAB_DIV(a, b) ((a) / (b))
-#else
+ * from __fdividef's 2^126 caveat. */
 #define SDFR_SLAB_DIV(a, b) __fdividef((a), (b))
-#endif
 #else
 #include <math.h>
 #define SDFR_LDG(p) (*(p))
@@ -80,14 +76,6 @@ struct Grid {
  */
 constexpr int kLayoutDense = 0;
 constexpr int kLayoutSkewed = 1;
-/* Z-PAIR (experimental, A/B of DESIGN.md section 5): a float2 per voxel, (v[x][y][z], v[x][y][min(z+1,R-1)]), so
- * that the 8 corners of a cell are 4 aligned 8-byte loads instead of 8 4-byte ones; pitches in float2 units
- * with pitch_y = 3, pitch_x = 9 (mod 16: 16 float2 per 128-byte line).  Twice the footprint of the grid. */
-constexpr int kLayoutZPair = 2;
-SDFR_HDC int zpair_pitch_y(int R) { return R + (((3 - R % 16) + 16) % 16); }
-SDFR_HDC int zpair_pitch_x(int R) {
-  return R * zpair_pitch_y(R) + (((9 - (R * zpair_pitch_y(R)) % 16) + 16) % 16);
-}
 
 SDFR_HDC int skew_pitch_y(int R) { return R + (((3 - R % 32) + 32) % 32); }
 SDFR_HDC int skew_pitch_x(int R) {
@@ -99,8 +87,8 @@ SDFR_HD Grid make_grid(int R, int layout = kLayoutDense) {
   G.R = R;
   G.R2 = R * R;
   G.Rm2 = R - 2;
-  G.py = layout == kLayoutSkewed ? skew_pitch_y(R) : (layout == kLayoutZPair ? zpair_pitch_y(R) : R);
-  G.px = layout == kLayoutSkewed ? skew_pitch_x(R) : (layout == kLayoutZPair ? zpair_pitch_x(R) : R * R);
+  G.py = layout == kLayoutSkewed ? skew_pitch_y(R) : R;
+  G.px = layout == kLayoutSkewed ? skew_pitch_x(R) : R * R;
   G.layout = layout;
   G.Rm1f = (float)(R - 1);
   G.h = (float)(2.0 / (double)(R - 1));
@@ -426,9 +414,9 @@ SDFR_HD bool ray_box(const Frame& F, const Ray& r, float& t_min, float& t_max) {
  * ~150 -> ~60 SASS instructions per ray; per-pixel set-up was 31 % of the fused kernel's instructions
  * (profiles/r02ag_ncu_fused_segments.txt).  The early exits of cu:171-189 can be taken at the end instead:
  * t_min only grows and t_max only shrinks over the slabs, so `t_min > t_max || t_max < 0` after any slab
- * implies the same after the last.  Host build / -DSDFR_EXACT_SLAB_DIV: the two separate tests above. */
+ * implies the same after the last.  Host build: the two separate tests above. */
 SDFR_HD bool ray_cull_and_box(const Frame& F, const Ray& r, float& t_min, float& t_max) {
-#if defined(__CUDA_ARCH__) && !defined(SDFR_EXACT_SLAB_DIV) && !defined(SDFR_SEPARATE_SLAB_TESTS)
+#if defined(__CUDA_ARCH__)
   const bool a0 = fabsf(r.dox) > 1e-20f, a1 = fabsf(r.doy) > 1e-20f, a2 = fabsf(r.doz) > 1e-20f;
   float i0, i1, i2;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(i0) : "f"(a0 ? r.dox : 1.0f));
@@ -501,17 +489,6 @@ struct Corners {
  * address computation and use immediate offsets (RT = 0: run-time pitches G.py / G.px). */
 template <int RT, int LT = kLayoutDense>
 SDFR_HD Corners gather(const float* __restrict__ g, const Grid& G, int ix, int iy, int iz) {
-#if defined(__CUDA_ARCH__)
-  if (RT > 0 && LT == kLayoutZPair) {
-    constexpr int PY2 = zpair_pitch_y(RT > 0 ? RT : 2), PX2 = zpair_pitch_x(RT > 0 ? RT : 2);
-    const float2* c2 = reinterpret_cast<const float2*>(g) + (ix * PX2 + iy * PY2 + iz);
-    const float2 a = __ldg(c2), b = __ldg(c2 + PY2), d = __ldg(c2 + PX2), e = __ldg(c2 + PX2 + PY2);
-    Corners kz;
-    kz.c000 = a.x; kz.c001 = a.y; kz.c010 = b.x; kz.c011 = b.y;
-    kz.c100 = d.x; kz.c101 = d.y; kz.c110 = e.x; kz.c111 = e.y;
-    return kz;
-  }
-#endif
   const int PY = RT > 0 ? (LT == kLayoutSkewed ? skew_pitch_y(RT) : RT) : G.py;
   const int PX = RT > 0 ? (LT == kLayoutSkewed ? skew_pitch_x(RT) : RT * RT) : G.px;
   const float* c = g + (ix * PX + iy * PY + iz);

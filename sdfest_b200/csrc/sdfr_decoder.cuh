@@ -483,20 +483,11 @@ struct ConvParams {
 
 /* Shared-memory geometry of one CTA: CC input channels of the (TX+2) x (TY+2) x (TZ+2) input tile,
  * z-pitch PZ a multiple of 4 floats so that staging and the inner loop use 128 / 64-bit accesses. */
-#ifndef SDFR_CONV_CC_ZR4
-#define SDFR_CONV_CC_ZR4 8 /* input channels staged per pass by the 32-deep tiles (tuning knob) */
-#endif
-#ifndef SDFR_CONV_FFMA2
-#define SDFR_CONV_FFMA2 1 /* packed fp32 multiply-adds (FFMA2) in the convolution's inner loop */
-#endif
-#ifndef SDFR_CONV_YR2_MAX_ACC
-#define SDFR_CONV_YR2_MAX_ACC 0 /* CO*ZR up to which a thread computes two output rows (tuning knob, off) */
-#endif
-template <int CO, int ZR, int YR = 1>
+template <int CO, int ZR>
 struct ConvTile {
-  static constexpr int K = 3, TX = 4, TY = 8 * YR, TZ = 8 * ZR;
+  static constexpr int K = 3, TX = 4, TY = 8, TZ = 8 * ZR;
   /* channels staged per pass: the tile must leave room for >= 3 CTAs per SM */
-  static constexpr int CC = YR == 2 ? 4 : (ZR == 4 ? SDFR_CONV_CC_ZR4 : 8);
+  static constexpr int CC = 8;
   static constexpr int IX = TX + K - 1, IY = TY + K - 1, IZ = TZ + K - 1;
   static constexpr int PZ = ((IZ + 3) / 4) * 4;
   static constexpr int CH = IX * IY * PZ; /* floats per staged channel */
@@ -514,17 +505,12 @@ struct ConvTile {
  * (8^3 -> 6^3: 2 tiles per volume, 128 CTAs of 9 k instructions per thread at 64 hypotheses --
  * one CTA per SM, latency-bound at 8 warps) this quadruples the resident warps without shrinking
  * the per-thread accumulator block (splitting the OUTPUT channels instead was measured slower). */
-/* YR = 2: a thread computes two adjacent output rows (y), sharing the 4 input rows they read and
- * every weight vector: shared-memory wavefronts per FFMA drop from 0.19 to 0.115 (the 32-deep tile is
- * co-limited by the LDS pipe at 69 % with the FMA pipe at 58 %, profiles/r01s_ncu_decoder.txt).
- * Measured (-DSDFR_CONV_YR2_MAX_ACC=16 / 32): no gain at 64 hypotheses -- 108 us either way for the
- * 8 -> 4 channel stage, 151 instead of 133 us for its data gradient with 64 accumulators; half as many,
- * twice as long CTAs quantise worse into waves of 3 CTAs per SM.  Left as a knob, off by default. */
-template <int CO, int ZR, bool DGRAD, int VEC, int KS = 1, int YR = 1>
-__global__ void __launch_bounds__(256, (CO * ZR * YR <= 16 ? 4 : (CO * ZR * YR <= 32 ? 3 : (CO * ZR * YR <= 64 ? 2 : 1))))
+/* A thread computing two adjacent output rows, sharing their input rows and weights, was measured slower
+ * (8 -> 4 channel stage: 118.8 against 100.4 us, profiles/r02ad_conv_ffma2_ab.json). */
+template <int CO, int ZR, bool DGRAD, int VEC, int KS = 1>
+__global__ void __launch_bounds__(256, (CO * ZR <= 16 ? 4 : (CO * ZR <= 32 ? 3 : (CO * ZR <= 64 ? 2 : 1))))
 sdfr_conv3_kernel(const __grid_constant__ ConvParams P) {
-  using T = ConvTile<CO, ZR, YR>;
-  constexpr int NZ = YR * ZR; /* accumulators per output channel: [row r][z i] at r * ZR + i */
+  using T = ConvTile<CO, ZR>;
   constexpr int K = 3, TX = T::TX, TY = T::TY, TZ = T::TZ, CC = T::CC;
   constexpr int IX = T::IX, IY = T::IY, PZ = T::PZ;
   extern __shared__ __align__(16) float conv_smem[];
@@ -548,18 +534,12 @@ sdfr_conv3_kernel(const __grid_constant__ ConvParams P) {
   /* Accumulators as float2 pairs over adjacent output channels: the weight vector of a tap arrives as
    * float4 = two aligned channel pairs, the input value is duplicated into a pair once per row, and every
    * multiply-add is one FFMA2 (fma.rn.f32x2, sm_100) -- two IEEE fp32 fmas per issue slot and per fma-pipe
-   * cycle, bit-identical to the scalar FFMAs (-DSDFR_CONV_FFMA2=0 builds those for the A/B). */
-#if SDFR_CONV_FFMA2
-  float2 acc2[CO / 2][NZ];
-#define SDFR_ACC(co, i) (((co) & 1) ? acc2[(co) >> 1][i].y : acc2[(co) >> 1][i].x)
-#else
-  float acc[CO][NZ];
-#define SDFR_ACC(co, i) acc[co][i]
-#endif
+   * cycle, bit-identical to scalar FFMAs. */
+  float2 acc2[CO / 2][ZR];
 #pragma unroll
-  for (int co = 0; co < CO; ++co)
+  for (int c2 = 0; c2 < CO / 2; ++c2)
 #pragma unroll
-    for (int i = 0; i < NZ; ++i) SDFR_ACC(co, i) = 0.0f;
+    for (int i = 0; i < ZR; ++i) acc2[c2][i] = make_float2(0.0f, 0.0f);
 
   const int ci_begin = kr * (CI / KS), ci_end = ci_begin + CI / KS; /* CI % KS == 0 (launcher) */
   for (int ci0 = ci_begin; ci0 < ci_end; ci0 += CC) {
@@ -618,108 +598,42 @@ sdfr_conv3_kernel(const __grid_constant__ ConvParams P) {
       ws[e] = v;
     }
     __syncthreads();
-    if constexpr (YR == 1) {
-      /* one row per (dx, dy) at a time: loading the three rows of a dx up front (as the YR = 2 path
-       * below must) costs the 8 -> 4 channel stage 12 us -- more live registers, later first FFMA */
-      for (int c = 0; c < nc; ++c) {
+    /* one row per (dx, dy) at a time: loading the three rows of a dx up front costs the 8 -> 4 channel
+     * stage 12 us -- more live registers, later first FFMA */
+    for (int c = 0; c < nc; ++c) {
 #pragma unroll
-        for (int dx = 0; dx < K; ++dx) {
+      for (int dx = 0; dx < K; ++dx) {
 #pragma unroll
-          for (int dy = 0; dy < K; ++dy) {
-            float v[ZR + K - 1];
-            const float* __restrict__ row = tile + ((c * IX + lx + dx) * IY + ly + dy) * PZ + z0;
-            if constexpr (ZR == 4) {
-              const float4 a = *reinterpret_cast<const float4*>(row);
-              const float2 e2 = *reinterpret_cast<const float2*>(row + 4);
-              v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = e2.x; v[5] = e2.y;
-            } else if constexpr (ZR == 2) {
-              const float2 a = *reinterpret_cast<const float2*>(row);
-              const float2 e2 = *reinterpret_cast<const float2*>(row + 2);
-              v[0] = a.x; v[1] = a.y; v[2] = e2.x; v[3] = e2.y;
-            } else {
+        for (int dy = 0; dy < K; ++dy) {
+          float v[ZR + K - 1];
+          const float* __restrict__ row = tile + ((c * IX + lx + dx) * IY + ly + dy) * PZ + z0;
+          if constexpr (ZR == 4) {
+            const float4 a = *reinterpret_cast<const float4*>(row);
+            const float2 e2 = *reinterpret_cast<const float2*>(row + 4);
+            v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = e2.x; v[5] = e2.y;
+          } else if constexpr (ZR == 2) {
+            const float2 a = *reinterpret_cast<const float2*>(row);
+            const float2 e2 = *reinterpret_cast<const float2*>(row + 2);
+            v[0] = a.x; v[1] = a.y; v[2] = e2.x; v[3] = e2.y;
+          } else {
 #pragma unroll
-              for (int i = 0; i < ZR + K - 1; ++i) v[i] = row[i];
-            }
-#if SDFR_CONV_FFMA2
-            float2 vv[ZR + K - 1];
-#pragma unroll
-            for (int i = 0; i < ZR + K - 1; ++i) vv[i] = make_float2(v[i], v[i]);
-#endif
-#pragma unroll
-            for (int dz = 0; dz < K; ++dz) {
-              const float4* __restrict__ wp =
-                  reinterpret_cast<const float4*>(ws + (c * 27 + (dx * K + dy) * K + dz) * CO);
-#pragma unroll
-              for (int c4 = 0; c4 < CO / 4; ++c4) {
-                const float4 w4 = wp[c4];
-#if SDFR_CONV_FFMA2
-                const float2 wa = make_float2(w4.x, w4.y), wb = make_float2(w4.z, w4.w);
-#pragma unroll
-                for (int i = 0; i < ZR; ++i) {
-                  acc2[2 * c4 + 0][i] = __ffma2_rn(wa, vv[i + dz], acc2[2 * c4 + 0][i]);
-                  acc2[2 * c4 + 1][i] = __ffma2_rn(wb, vv[i + dz], acc2[2 * c4 + 1][i]);
-                }
-#else
-#pragma unroll
-                for (int i = 0; i < ZR; ++i) {
-                  acc[4 * c4 + 0][i] = fmaf(w4.x, v[i + dz], acc[4 * c4 + 0][i]);
-                  acc[4 * c4 + 1][i] = fmaf(w4.y, v[i + dz], acc[4 * c4 + 1][i]);
-                  acc[4 * c4 + 2][i] = fmaf(w4.z, v[i + dz], acc[4 * c4 + 2][i]);
-                  acc[4 * c4 + 3][i] = fmaf(w4.w, v[i + dz], acc[4 * c4 + 3][i]);
-                }
-#endif
-              }
-            }
+            for (int i = 0; i < ZR + K - 1; ++i) v[i] = row[i];
           }
-        }
-      }
-    } else {
-      for (int c = 0; c < nc; ++c) {
+          float2 vv[ZR + K - 1];
 #pragma unroll
-        for (int dx = 0; dx < K; ++dx) {
-          float v[YR + K - 1][ZR + K - 1]; /* the input rows this thread's YR output rows read */
+          for (int i = 0; i < ZR + K - 1; ++i) vv[i] = make_float2(v[i], v[i]);
 #pragma unroll
-          for (int ry = 0; ry < YR + K - 1; ++ry) {
-            const float* __restrict__ row = tile + ((c * IX + lx + dx) * IY + ly * YR + ry) * PZ + z0;
-            if constexpr (ZR == 4) {
-              const float4 a = *reinterpret_cast<const float4*>(row);
-              const float2 e2 = *reinterpret_cast<const float2*>(row + 4);
-              v[ry][0] = a.x; v[ry][1] = a.y; v[ry][2] = a.z; v[ry][3] = a.w; v[ry][4] = e2.x; v[ry][5] = e2.y;
-            } else if constexpr (ZR == 2) {
-              const float2 a = *reinterpret_cast<const float2*>(row);
-              const float2 e2 = *reinterpret_cast<const float2*>(row + 2);
-              v[ry][0] = a.x; v[ry][1] = a.y; v[ry][2] = e2.x; v[ry][3] = e2.y;
-            } else {
+          for (int dz = 0; dz < K; ++dz) {
+            const float4* __restrict__ wp =
+                reinterpret_cast<const float4*>(ws + (c * 27 + (dx * K + dy) * K + dz) * CO);
 #pragma unroll
-              for (int i = 0; i < ZR + K - 1; ++i) v[ry][i] = row[i];
-            }
-          }
+            for (int c4 = 0; c4 < CO / 4; ++c4) {
+              const float4 w4 = wp[c4];
+              const float2 wa = make_float2(w4.x, w4.y), wb = make_float2(w4.z, w4.w);
 #pragma unroll
-          for (int dy = 0; dy < K; ++dy) {
-#pragma unroll
-            for (int dz = 0; dz < K; ++dz) {
-              const float4* __restrict__ wp =
-                  reinterpret_cast<const float4*>(ws + (c * 27 + (dx * K + dy) * K + dz) * CO);
-#pragma unroll
-              for (int c4 = 0; c4 < CO / 4; ++c4) {
-                const float4 w4 = wp[c4];
-#pragma unroll
-                for (int r = 0; r < YR; ++r) {
-#pragma unroll
-                  for (int i = 0; i < ZR; ++i) {
-                    const float x = v[r + dy][i + dz];
-#if SDFR_CONV_FFMA2
-                    const float2 xx = make_float2(x, x);
-                    acc2[2 * c4 + 0][r * ZR + i] = __ffma2_rn(make_float2(w4.x, w4.y), xx, acc2[2 * c4 + 0][r * ZR + i]);
-                    acc2[2 * c4 + 1][r * ZR + i] = __ffma2_rn(make_float2(w4.z, w4.w), xx, acc2[2 * c4 + 1][r * ZR + i]);
-#else
-                    acc[4 * c4 + 0][r * ZR + i] = fmaf(w4.x, x, acc[4 * c4 + 0][r * ZR + i]);
-                    acc[4 * c4 + 1][r * ZR + i] = fmaf(w4.y, x, acc[4 * c4 + 1][r * ZR + i]);
-                    acc[4 * c4 + 2][r * ZR + i] = fmaf(w4.z, x, acc[4 * c4 + 2][r * ZR + i]);
-                    acc[4 * c4 + 3][r * ZR + i] = fmaf(w4.w, x, acc[4 * c4 + 3][r * ZR + i]);
-#endif
-                  }
-                }
+              for (int i = 0; i < ZR; ++i) {
+                acc2[2 * c4 + 0][i] = __ffma2_rn(wa, vv[i + dz], acc2[2 * c4 + 0][i]);
+                acc2[2 * c4 + 1][i] = __ffma2_rn(wb, vv[i + dz], acc2[2 * c4 + 1][i]);
               }
             }
           }
@@ -733,21 +647,25 @@ sdfr_conv3_kernel(const __grid_constant__ ConvParams P) {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     __syncthreads(); /* everyone is done with the tile: its memory becomes the exchange buffer */
-    float* red = conv_smem; /* [CO * NZ][256] */
+    float* red = conv_smem; /* [CO * ZR][256] */
     if (kr != 0) {
 #pragma unroll
       for (int co = 0; co < CO; ++co)
 #pragma unroll
-        for (int i = 0; i < NZ; ++i) red[(co * NZ + i) * 256 + threadIdx.x] = SDFR_ACC(co, i);
+        for (int i = 0; i < ZR; ++i)
+          red[(co * ZR + i) * 256 + threadIdx.x] = (co & 1) ? acc2[co >> 1][i].y : acc2[co >> 1][i].x;
     }
     cluster.sync();
     if (kr == 0) {
       for (int r = 1; r < KS; ++r) {
         const float* __restrict__ peer = cluster.map_shared_rank(red, r);
 #pragma unroll
-        for (int co = 0; co < CO; ++co)
+        for (int c2 = 0; c2 < CO / 2; ++c2)
 #pragma unroll
-          for (int i = 0; i < NZ; ++i) SDFR_ACC(co, i) += peer[(co * NZ + i) * 256 + threadIdx.x];
+          for (int i = 0; i < ZR; ++i) {
+            acc2[c2][i].x += peer[(2 * c2 * ZR + i) * 256 + threadIdx.x];
+            acc2[c2][i].y += peer[((2 * c2 + 1) * ZR + i) * 256 + threadIdx.x];
+          }
       }
     }
     cluster.sync(); /* peers keep their shared memory alive until the leader has read it */
@@ -757,39 +675,35 @@ sdfr_conv3_kernel(const __grid_constant__ ConvParams P) {
   const int ox = X0 + lx;
   if (ox >= n_out) return;
   const size_t out_vol = (size_t)n_out * n_out * n_out;
+  const int oy = Y0 + ly;
+  if (oy >= n_out) return;
 #pragma unroll
-  for (int r = 0; r < YR; ++r) {
-    const int oy = Y0 + ly * YR + r;
-    if (oy >= n_out) continue;
+  for (int co = 0; co < CO; ++co) {
+    const float bias = (!DGRAD && P.bias) ? __ldg(P.bias + co0 + co) : 0.0f;
+    float* __restrict__ o = P.out + ((size_t)b * COT + co0 + co) * out_vol + ((size_t)ox * n_out + oy) * n_out;
 #pragma unroll
-    for (int co = 0; co < CO; ++co) {
-      const float bias = (!DGRAD && P.bias) ? __ldg(P.bias + co0 + co) : 0.0f;
-      float* __restrict__ o = P.out + ((size_t)b * COT + co0 + co) * out_vol + ((size_t)ox * n_out + oy) * n_out;
-#pragma unroll
-      for (int i = 0; i < ZR; ++i) {
-        const int oz = Z0 + z0 + i;
-        if (oz < n_out) {
-          float v = SDFR_ACC(co, r * ZR + i) + bias;
-          if (!DGRAD && P.relu) v = v > 0.0f ? v : 0.0f;
-          o[oz] = v;
-        }
+    for (int i = 0; i < ZR; ++i) {
+      const int oz = Z0 + z0 + i;
+      if (oz < n_out) {
+        float v = ((co & 1) ? acc2[co >> 1][i].y : acc2[co >> 1][i].x) + bias;
+        if (!DGRAD && P.relu) v = v > 0.0f ? v : 0.0f;
+        o[oz] = v;
       }
     }
   }
 }
-#undef SDFR_ACC
 
-template <int CO, int ZR, bool DGRAD, int VEC, int KS = 1, int YR = 1>
+template <int CO, int ZR, bool DGRAD, int VEC, int KS = 1>
 int launch_conv3_v(ConvParams P, int batch, cudaStream_t s) {
-  using T = ConvTile<CO, ZR, YR>;
+  using T = ConvTile<CO, ZR>;
   const int tiles_x = (P.n_out + T::TX - 1) / T::TX;
   P.tiles_y = (P.n_out + T::TY - 1) / T::TY;
   P.tiles_z = (P.n_out + T::TZ - 1) / T::TZ;
   const int per_cta = P.CI / KS;
   P.cc = per_cta < T::CC ? per_cta : T::CC;
   size_t smem = T::bytes(P.cc);
-  if (KS > 1 && smem < sizeof(float) * CO * ZR * YR * 256) smem = sizeof(float) * CO * ZR * YR * 256;
-  auto kernel = sdfr_conv3_kernel<CO, ZR, DGRAD, VEC, KS, YR>;
+  if (KS > 1 && smem < sizeof(float) * CO * ZR * 256) smem = sizeof(float) * CO * ZR * 256;
+  auto kernel = sdfr_conv3_kernel<CO, ZR, DGRAD, VEC, KS>;
   if (smem > 48 * 1024) {
     const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return fail((int)e, "conv3d: shared memory opt-in failed");
@@ -835,11 +749,10 @@ int launch_conv3_t(const ConvParams& P, int batch, cudaStream_t s) {
       if (P.n_in % 2 == 0 && (a & 7) == 0) return launch_conv3_v<CO, ZR, DGRAD, 2, 4>(P, batch, s);
     }
   }
-  constexpr int YR = (ZR >= 2 && CO * ZR <= SDFR_CONV_YR2_MAX_ACC) ? 2 : 1;
   if constexpr (!DGRAD)
-    if (P.n_in % 4 == 0 && (a & 15) == 0) return launch_conv3_v<CO, ZR, DGRAD, 4, 1, YR>(P, batch, s);
-  if (P.n_in % 2 == 0 && (a & 7) == 0) return launch_conv3_v<CO, ZR, DGRAD, 2, 1, YR>(P, batch, s);
-  return launch_conv3_v<CO, ZR, DGRAD, 1, 1, YR>(P, batch, s);
+    if (P.n_in % 4 == 0 && (a & 15) == 0) return launch_conv3_v<CO, ZR, DGRAD, 4>(P, batch, s);
+  if (P.n_in % 2 == 0 && (a & 7) == 0) return launch_conv3_v<CO, ZR, DGRAD, 2>(P, batch, s);
+  return launch_conv3_v<CO, ZR, DGRAD, 1>(P, batch, s);
 }
 
 /* z-extent of the CTA tile (8 * ZR) follows the volume: 32 for n_out > 16, 16 for > 8, else 8 --

@@ -29,7 +29,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "../../include/sdfrender.h"
@@ -345,13 +344,7 @@ __device__ __forceinline__ void scatter_sdf_warp(float* __restrict__ gs, const G
     }
     if (merge && !lower) alive = false;
   }
-#ifdef SDFR_AB_DROP_RED
-  /* A/B only (scripts/ab/ab_variants.sh): everything but the RED.ADDs themselves -- the upper bound of
-   * what any privatisation of the scatter could save */
-  if (alive && w[0] == 1.2345e30f) scatter_sdf<RT>(gs, G, base, w);
-#else
   if (alive) scatter_sdf<RT>(gs, G, base, w);
-#endif
 }
 
 /* Pose gradients of a CTA.  Every thread keeps its 13 moment sums (sdfr_core.cuh:
@@ -486,11 +479,9 @@ __device__ __forceinline__ void scale_sdf_grads(float* __restrict__ gs, const Ce
  * factor upstream/n_overlap is only known once all pixels are done and is applied afterwards by
  * sdfr_scale_grads -- every gradient is linear in it).
  * ---------------------------------------------------------------------------------------- */
-#ifndef SDFR_FWD_BLOCKS
-#define SDFR_FWD_BLOCKS 5 /* resident CTAs per SM the forward kernels are register-budgeted for */
-#endif
+constexpr int kFwdBlocks = 5; /* resident CTAs per SM the forward kernels are register-budgeted for */
 template <int RT, int LT, int MODE, bool STATS, bool WANT_SDF, bool WANT_POSE>
-__global__ void __launch_bounds__(kThreads, SDFR_FWD_BLOCKS)
+__global__ void __launch_bounds__(kThreads, kFwdBlocks)
 sdfr_forward_kernel(const __grid_constant__ FwdParams P) {
   extern __shared__ float tables[];
   __shared__ Frame Fs;
@@ -644,13 +635,8 @@ sdfr_forward_kernel(const __grid_constant__ FwdParams P) {
                                                               (P.flags & SDFR_SDF_GRAD_EXACT) != 0, base, w8, m);
           if (WANT_POSE) moments_add(acc_s, m);
         }
-        if (WANT_SDF) {
-#ifdef SDFR_NO_WARP_AGGREGATION
-          if (sgn != 0.0f) scatter_sdf<RT>(P.grad_sdf + (size_t)b * P.grad_sdf_stride, Gc, base, w8);
-#else
+        if (WANT_SDF)
           scatter_sdf_warp<RT>(P.grad_sdf + (size_t)b * P.grad_sdf_stride, Gc, base, w8, sgn != 0.0f, lane);
-#endif
-        }
       }
       if (lane == 0) q = atomicAdd(&next_q, 1);
       q = __shfl_sync(kFull, q, 0);
@@ -692,11 +678,9 @@ sdfr_forward_kernel(const __grid_constant__ FwdParams P) {
 /* Register budget of the backward kernels: the SDF+pose variant needs ~80 registers; squeezed
  * into 64 (4 CTAs/SM) it spills, and the spill traffic (7 M write sectors per launch at C2,
  * profiles/r01d_bwd_ncu.txt) made it 4x slower than either single-purpose variant. */
-#ifndef SDFR_BWD_BLOCKS
-#define SDFR_BWD_BLOCKS 4
-#endif
+constexpr int kBwdBlocks = 4;
 template <int RT, int LT, int MODE, bool WANT_SDF, bool WANT_POSE>
-__global__ void __launch_bounds__(kThreads, SDFR_BWD_BLOCKS)
+__global__ void __launch_bounds__(kThreads, kBwdBlocks)
 sdfr_backward_kernel(const __grid_constant__ BwdParams P) {
   extern __shared__ float tables[];
   __shared__ Frame Fs;
@@ -1217,22 +1201,6 @@ sdfr_bounds_from_minima_kernel(const float* __restrict__ minima, int R, const fl
   }
 }
 
-/* Dense [R][R][R] -> z-pair copy (sdfr_core.cuh: kLayoutZPair): one float2 per voxel. */
-__global__ void __launch_bounds__(256)
-sdfr_zpair_kernel(const float* __restrict__ src, long long src_stride, float* __restrict__ dst,
-                  long long dst_stride, int R, int py2, int px2) {
-  const int b = blockIdx.y;
-  const float* __restrict__ s = src + (size_t)b * src_stride;
-  float2* __restrict__ d = reinterpret_cast<float2*>(dst + (size_t)b * dst_stride);
-  const int n = R * R * R;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const int row = i / R, z = i - row * R;
-    const int ix = row / R, iy = row - ix * R;
-    const float v0 = __ldg(s + i), v1 = z + 1 < R ? __ldg(s + i + 1) : v0;
-    d[(size_t)ix * px2 + iy * py2 + z] = make_float2(v0, v1);
-  }
-}
-
 /* Dense [R][R][R] -> skewed pitched copy (sdfr_core.cuh: kLayoutSkewed).  One warp per (x,y)
  * row: coalesced reads, coalesced (unaligned) writes; the padding is never read. */
 __global__ void __launch_bounds__(256)
@@ -1267,10 +1235,8 @@ sdfr_skew_kernel(const float* __restrict__ src, long long src_stride, float* __r
  * Host side
  * ---------------------------------------------------------------------------------------- */
 int check_common(const float* sdf, int R, long long sdf_stride, int layout, const float* pos,
-                 const float* quat, const float* inv_scale, int batch, int W, int H, bool allow_zpair = false) {
-  if (layout != SDFR_LAYOUT_DENSE && layout != SDFR_LAYOUT_SKEWED &&
-      !(allow_zpair && layout == SDFR_LAYOUT_ZPAIR && R == 64))
-    return fail(SDFR_E_FLAGS, "unknown sdf_layout (the experimental z-pair layout: resolution 64 only)");
+                 const float* quat, const float* inv_scale, int batch, int W, int H) {
+  if (layout != SDFR_LAYOUT_DENSE && layout != SDFR_LAYOUT_SKEWED) return fail(SDFR_E_FLAGS, "unknown sdf_layout");
   if (batch < 0 || W < 0 || H < 0) return fail(SDFR_E_SHAPE, "negative batch/width/height");
   if (R < 2 || R > 1024) return fail(SDFR_E_SHAPE, "resolution must be in [2, 1024]");
   if (sdf_stride < 0) return fail(SDFR_E_SHAPE, "negative sdf_stride");
@@ -1316,11 +1282,7 @@ int ctas_per_hypothesis(int batch, int W, int H) {
   /* 16 CTAs per SM in total for larger batches (measured at 64 hypotheses, profiles/r01zp_micro.json
    * c2_cta_sweep: 2368 CTAs beat 4736 by 2 % forward / fused and 6 % backward); small batches keep 32
    * so that a single large frame still gets one CTA per tile */
-  long long target = (long long)sm_count() * (batch >= 16 ? 16 : 32);
-  if (const char* env = getenv("SDFR_TARGET_CTAS")) { /* tuning knob, see scripts/gpu_micro.py */
-    const long long v = atoll(env);
-    if (v > 0) target = v;
-  }
+  const long long target = (long long)sm_count() * (batch >= 16 ? 16 : 32);
   long long g = (target + batch - 1) / batch;
   if (g > n_tiles) g = n_tiles;
   if (g > 65535) g = 65535;
@@ -1375,14 +1337,6 @@ int launch_forward(FwdParams P, int batch, cudaStream_t s) {
   for (int z0 = 0; z0 < batch; z0 += 65535) {
     P.z_offset = z0;
     const dim3 grid(G, batch - z0 < 65535 ? batch - z0 : 65535);
-    if (P.grid.layout == kLayoutZPair) { /* experimental: the compare entry points at 64^3 only */
-      if constexpr (MODE >= 1 && !STATS) {
-        launch_forward_rt<64, kLayoutZPair, MODE, STATS>(P, grid, smem, s);
-        continue;
-      } else {
-        return fail(SDFR_E_FLAGS, "the z-pair layout is only wired into sdfr_compare_forward / sdfr_compare_fused");
-      }
-    }
 #define SDFR_CALL(RT, LT) launch_forward_rt<RT, LT, MODE, STATS>(P, grid, smem, s)
     SDFR_DISPATCH_RT_LT(P.grid.R, skewed, SDFR_CALL);
 #undef SDFR_CALL
@@ -1402,12 +1356,12 @@ void launch_backward_rt(BwdParams& P, dim3 grid, size_t smem, bool want_sdf, boo
 }
 
 /*
- * The backward is launched in chunks of hypotheses whose working set (gradient grid, SDF grid,
- * depth and upstream images) fits comfortably in L2, each chunk's gradient grids being cleared
- * right before its kernel: the scattered RED.ADDs then hit lines that are still L2-resident.
- * Clearing all grids up front lets the streaming reads of the first hypotheses evict the zeroed
- * lines of the later ones, and every RED becomes a 32-byte read-modify-write against HBM
- * (measured at B = 64, 64^3, 640x480: 457 us against 105 us for the pose gradients alone).
+ * The backward is launched once per slice of at most 65535 hypotheses (the gridDim.y limit).  With
+ * ZERO_GRADS, the per-hypothesis gradient grids of a slice are cleared right before its launch, so
+ * that the scattered RED.ADDs hit zeroed lines that are still L2-resident; a shared gradient grid
+ * is cleared once before the first slice.  The clear stays next to the launch: when the zeroed
+ * lines are evicted before the kernel runs, every RED becomes a 32-byte read-modify-write against
+ * HBM (measured at B = 64, 64^3, 640x480: 457 us against 105 us for the pose gradients alone).
  */
 template <int MODE>
 int launch_backward(BwdParams P, int batch, bool zero_sdf, cudaStream_t s) {
@@ -1418,24 +1372,12 @@ int launch_backward(BwdParams P, int batch, bool zero_sdf, cudaStream_t s) {
   const size_t smem = table_bytes(P.cam.W, P.cam.H);
   P.use_tables = smem != 0;
   const bool skewed = P.grid.layout == kLayoutSkewed;
-  if (P.grid.layout == kLayoutZPair) return fail(SDFR_E_FLAGS, "the z-pair layout is not wired into the backward entry points");
   const size_t grid_bytes = sizeof(float) * (size_t)P.grid.R * P.grid.R * P.grid.R;
-  int chunk = batch;
-  if (want_sdf && P.grad_sdf_stride != 0) {
-    const size_t per_hyp = grid_bytes + (P.sdf_stride != 0 ? grid_bytes : 0) +
-                           2 * sizeof(float) * (size_t)P.cam.W * P.cam.H;
-    size_t budget_mb = 0; /* 0 = one launch for the whole batch */
-    if (const char* env = getenv("SDFR_BWD_CHUNK_MB")) budget_mb = (size_t)atoll(env);
-    if (budget_mb > 0) {
-      chunk = (int)((budget_mb << 20) / per_hyp);
-      chunk = chunk < 1 ? 1 : (chunk > batch ? batch : chunk);
-    }
-  } else if (zero_sdf && want_sdf) { /* one shared gradient grid */
+  if (zero_sdf && want_sdf && P.grad_sdf_stride == 0) { /* one shared gradient grid */
     if (int rc = zero_async(P.grad_sdf, grid_bytes, s)) return rc;
   }
-  if (chunk > 65535) chunk = 65535;
-  for (int z0 = 0; z0 < batch; z0 += chunk) {
-    const int nz = batch - z0 < chunk ? batch - z0 : chunk;
+  for (int z0 = 0; z0 < batch; z0 += 65535) {
+    const int nz = batch - z0 < 65535 ? batch - z0 : 65535;
     if (zero_sdf && want_sdf && P.grad_sdf_stride != 0) {
       if ((size_t)P.grad_sdf_stride * sizeof(float) == grid_bytes) {
         if (int rc = zero_async(P.grad_sdf + (size_t)z0 * P.grad_sdf_stride, grid_bytes * nz, s))
@@ -1621,7 +1563,7 @@ int sdfr_compare_forward(const float* sdf, int R, long long sdf_stride, int layo
                          const float* depth_obs, long long obs_stride, float* depth,
                          float* loss_sum, float* n_overlap, unsigned flags,
                          const sdfr_cell_bounds* bounds, void* stream) {
-  if (int rc = check_common(sdf, R, sdf_stride, layout, pos, quat, inv_scale, batch, W, H, true)) return rc;
+  if (int rc = check_common(sdf, R, sdf_stride, layout, pos, quat, inv_scale, batch, W, H)) return rc;
   if (flags & ~SDFR_ZERO_GRADS) return fail(SDFR_E_FLAGS, "unknown flag bits");
   if (obs_stride < 0) return fail(SDFR_E_SHAPE, "negative obs_stride");
   if (batch == 0) return 0;
@@ -1681,7 +1623,7 @@ static int compare_fused_impl(const float* sdf, int R, long long sdf_stride, int
                               float* loss_sum, float* n_overlap, float rel_threshold, float* n_inlier,
                               float* gs, long long gs_stride, float* gp, float* gq, float* gi,
                               unsigned flags, const sdfr_cell_bounds* bounds, void* stream) {
-  if (int rc = check_common(sdf, R, sdf_stride, layout, pos, quat, inv_scale, batch, W, H, true)) return rc;
+  if (int rc = check_common(sdf, R, sdf_stride, layout, pos, quat, inv_scale, batch, W, H)) return rc;
   if (int rc = check_backward_outputs(flags, gs, gs_stride, gp, gq, gi)) return rc;
   if (obs_stride < 0) return fail(SDFR_E_SHAPE, "negative obs_stride");
   if ((flags & SDFR_GRAD_SDF) && gs_stride == 0 && batch > 1)
@@ -1914,30 +1856,6 @@ int sdfr_skew_grids_bounds(const float* sdf, int R, long long sdf_stride, int ba
   if (sdf_stride == 0 && batch > 1) skewed_stride = 0; /* one shared grid: one skewed copy */
   return launch_bounds_scan(sdf, R, sdf_stride, SDFR_LAYOUT_DENSE, pos, inv_scale, batch, threshold, bounds, skewed,
                             skewed_stride, (cudaStream_t)stream);
-}
-
-int sdfr_zpair_elems(int R, long long* elems) {
-  if (R < 2 || R > 1024) return fail(SDFR_E_SHAPE, "resolution must be in [2, 1024]");
-  if (elems) *elems = 2ll * R * zpair_pitch_x(R);
-  return 0;
-}
-
-int sdfr_zpair_grids(const float* sdf, int R, long long sdf_stride, int batch, float* zpair,
-                     long long zpair_stride, void* stream) {
-  if (R < 2 || R > 1024) return fail(SDFR_E_SHAPE, "resolution must be in [2, 1024]");
-  if (batch < 0 || sdf_stride < 0) return fail(SDFR_E_SHAPE, "negative batch or sdf_stride");
-  if (batch == 0) return 0;
-  if (!sdf || !zpair) return fail(SDFR_E_NULL, "NULL grid pointer");
-  if (zpair_stride < 2ll * R * zpair_pitch_x(R)) return fail(SDFR_E_SHAPE, "zpair_stride smaller than sdfr_zpair_elems");
-  const long long work = (long long)R * R * R;
-  const int gx = (int)((work + 255) / 256 < 2048 ? (work + 255) / 256 : 2048);
-  for (int z0 = 0; z0 < batch; z0 += 65535) {
-    const int nz = batch - z0 < 65535 ? batch - z0 : 65535;
-    sdfr_zpair_kernel<<<dim3(gx, nz), 256, 0, (cudaStream_t)stream>>>(
-        sdf + (size_t)z0 * sdf_stride, sdf_stride, zpair + (size_t)z0 * zpair_stride, zpair_stride, R,
-        zpair_pitch_y(R), zpair_pitch_x(R));
-  }
-  return check_launch("sdfr_zpair_kernel");
 }
 
 int sdfr_skewed_pitches(int R, int* pitch_y, int* pitch_x, long long* elems) {

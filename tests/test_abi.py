@@ -102,9 +102,9 @@ def test_skewed_layout_geometry():
     assert lib.sdfr_forward(None, 4, 0, 7, None, None, None, 1, *cam, 0.01, None, None, None) == -3
 
 
-def test_argument_errors_of_the_round_two_entry_points_need_no_gpu():
-    """Views, point constraint, slab minima, scale-with-bounds, tail-with-bounds, z-pair: empty work is a no-op,
-    NULL / bad sizes are reported before anything is launched."""
+def test_argument_errors_of_the_round_two_entry_points_and_an_unknown_layout_need_no_gpu():
+    """Views, point constraint, slab minima, scale-with-bounds, tail-with-bounds, compare layout: empty work is a
+    no-op, NULL / bad sizes and unknown layouts are reported before anything is launched."""
     import ctypes
 
     lib = _lib.lib()
@@ -135,17 +135,13 @@ def test_argument_errors_of_the_round_two_entry_points_need_no_gpu():
                                                 None, None) == -1
     assert lib.sdfr_decoder_tail_forward_bounds(None, 40, 30, None, None, None, 2, 64, None, 0, 0, None, None, 0.005,
                                                 None, None) == -2
-    n = ctypes.c_longlong(0)
-    assert lib.sdfr_zpair_elems(64, ctypes.byref(n)) == 0 and n.value == 2 * 64 * (64 * 67 + 9)
-    assert lib.sdfr_zpair_grids(None, 64, 0, 0, None, 0, None) == 0
-    assert lib.sdfr_zpair_grids(None, 64, 0, 1, None, 0, None) == -1
     cam = (8, 8, 4.0, 4.0, 4.0, 4.0)
-    # the experimental z-pair layout is refused everywhere but the compare entry points at 64^3
+    # layout id 2 (the removed z-pair layout) is refused like any other unknown id, also at 64^3
     assert lib.sdfr_forward(None, 64, 0, 2, None, None, None, 1, *cam, 0.01, None, None, None) == -3
     assert lib.sdfr_compare_forward(None, 32, 0, 2, None, None, None, 1, *cam, 0.01, None, 0, None, None, None, 0,
                                     None, None) == -3
     assert lib.sdfr_compare_forward(None, 64, 0, 2, None, None, None, 1, *cam, 0.01, None, 0, None, None, None, 0,
-                                    None, None) == -1  # accepted layout, NULL inputs
+                                    None, None) == -3
 
 
 def test_missing_library_fails_loudly(monkeypatch, tmp_path):
