@@ -96,6 +96,8 @@ struct FwdParams {
   float* __restrict__ depth;  // [B,H,W]
   int z_offset;               // first hypothesis of this launch (gridDim.y chunking)
   int use_tables;             // ray tables fit in shared memory
+  int steal;                  // more CTAs than fit at once: CTAs render unlaunched CTAs' items (WorkSteal)
+  int image_tables;           // use_tables, steal and several tiles per CTA: ray tables of the whole image, once
   // compare
   const float* __restrict__ depth_obs;
   long long obs_stride;
@@ -213,8 +215,9 @@ __device__ __forceinline__ float warp_sum(float v) {
  * Work decomposition of the batched kernels.
  *
  * grid = (G, hypotheses): G persistent CTAs per hypothesis.  A CTA builds the hypothesis' Frame
- * and the ray tables ONCE, then walks the 32x8-pixel tiles g, g+G, g+2G, ... of that hypothesis
- * without any further barrier: tiles outside the projected box are only zero-filled, tiles
+ * and the ray tables ONCE (the forward kernels: once per logical CTA, and a resident CTA renders
+ * several logical CTAs when it can steal them, see WorkSteal), then walks the 32x8-pixel tiles
+ * g, g+G, g+2G, ... of that hypothesis without any further barrier: tiles outside the projected box are only zero-filled, tiles
  * inside are traced.  Per-pixel results that need a reduction (loss sums, pose gradients,
  * counters) accumulate in registers across the CTA's tiles and are reduced once at the end.
  * (Round 1 first shipped one CTA per tile: 76 800 CTAs with a prologue + barrier each -- ncu
@@ -265,11 +268,13 @@ __device__ __forceinline__ Tiling make_tiling(const Frame& F, const Camera& cam)
   return T;
 }
 
-/* CTA prologue: Frame by warp 0, then the ray tables (double-precision divisions as in
- * cu:146-147, amortised over all tiles of the CTA).  When the CTA owns at most one tile of the
- * box (small batches: G >= number of box tiles) only that tile's 32 + 8 entries are built. */
+/* CTA prologue of logical CTA (g, b): Frame by warp 0, then -- with fill_tables -- the ray tables
+ * (double-precision divisions as in cu:146-147, amortised over all tiles of the CTA).  When the CTA
+ * owns at most one tile of the box (small batches: G >= number of box tiles) only that tile's
+ * 32 + 8 entries are built.  Without fill_tables the tables are either unused or already hold the
+ * whole image (fill_image_tables). */
 __device__ __forceinline__ Tiling cta_prologue(Frame& Fs, HullEdge* edges, float* tables,
-                                               bool use_tables, const Pose& pose, int b,
+                                               bool fill_tables, const Pose& pose, int g, int b,
                                                const Camera& cam, float*& colx, float*& rowy) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == 0) build_frame(Fs, edges, pose, b, cam, lane);
@@ -277,13 +282,13 @@ __device__ __forceinline__ Tiling cta_prologue(Frame& Fs, HullEdge* edges, float
   Tiling T = make_tiling(Fs, cam);
   colx = tables;
   rowy = tables + T.tiles_x * kTileW;
-  if (use_tables) {
+  if (fill_tables) {
     const int n_rect = T.rtw * T.rth;
     int ncol = T.rtw * kTileW, nrow = T.rth * kTileH;
-    if (n_rect <= (int)gridDim.x) { /* this CTA traces tile blockIdx.x of the box, or nothing */
-      if ((int)blockIdx.x < n_rect) {
-        const int ty = (int)blockIdx.x / T.rtw;
-        T.tab_x0 = T.rtx0 + ((int)blockIdx.x - ty * T.rtw);
+    if (n_rect <= (int)gridDim.x) { /* this CTA traces tile g of the box, or nothing */
+      if (g < n_rect) {
+        const int ty = g / T.rtw;
+        T.tab_x0 = T.rtx0 + (g - ty * T.rtw);
         T.tab_y0 = T.rty0 + ty;
         ncol = kTileW;
         nrow = kTileH;
@@ -302,6 +307,101 @@ __device__ __forceinline__ Tiling cta_prologue(Frame& Fs, HullEdge* edges, float
     __syncthreads();
   }
   return T;
+}
+
+/* Ray tables of the whole image: they depend on the camera only, so a CTA that renders several
+ * logical CTAs (WorkSteal) builds them once.  The caller synchronises before the first read. */
+__device__ __forceinline__ void fill_image_tables(float* tables, const Camera& cam) {
+  const int ncol = (cam.W + kTileW - 1) / kTileW * kTileW, nrow = (cam.H + kTileH - 1) / kTileH * kTileH;
+  for (int i = threadIdx.x; i < ncol; i += kThreads) tables[i] = pixel_dx(i, cam.cx, cam.fx);
+  for (int i = threadIdx.x; i < nrow; i += kThreads) tables[ncol + i] = pixel_dy(i, cam.cy, cam.fy);
+}
+
+/*
+ * Work stealing by cluster launch control (sm_100, PTX clusterlaunchcontrol.*): a CTA that has
+ * finished its logical CTA cancels one that the hardware has not launched yet and renders that one
+ * itself, so the per-CTA fixed costs are paid about once per resident CTA.  Nothing lives in global
+ * memory: no counter to reset between graph replays, nothing shared between two launches in flight.
+ * The first warp that finds the work list of the current item empty issues the request for the next
+ * one (the answer arrives while the other warps finish; issued at the start of the item instead, a
+ * busy CTA reserved work that a CTA finishing sooner could have started: fused launch +2 us instead
+ * of -10 us, DESIGN.md section 5).  Thread 0 waits on the mbarrier at the end of the item and
+ * publishes the next item in `next_g`, `next_b` (next_g < 0: no CTA left to take, the CTA exits).
+ * A failed request is never followed by another one (undefined in the PTX ISA): the loop ends on
+ * it.  The current item is
+ * copied to `g`, `b` at the start of each item and read back from there where it is needed (item_g,
+ * item_b): blockIdx was a special register that ptxas re-read at will, a loop variable would be two
+ * more registers live across the march.
+ */
+struct WorkSteal {
+  alignas(16) unsigned long long response[2]; /* try_cancel response, written by the async proxy */
+  unsigned long long bar;                      /* mbarrier: one arrival + 16 transaction bytes per request */
+  unsigned phase;                              /* parity of the request in flight (thread 0 only) */
+  int g, b;                                    /* current logical CTA: tile group, hypothesis (+ z_offset) */
+  int next_g, next_b;                          /* the one after it: blockIdx.x, blockIdx.y */
+  int requested;                               /* the request for next_g / next_b has been issued */
+};
+
+__device__ __forceinline__ int item_g(const WorkSteal& ws) { return *reinterpret_cast<const volatile int*>(&ws.g); }
+__device__ __forceinline__ int item_b(const WorkSteal& ws) { return *reinterpret_cast<const volatile int*>(&ws.b); }
+
+__device__ __forceinline__ void steal_init(WorkSteal& ws) {
+  if (threadIdx.x == 0) {
+    ws.next_g = blockIdx.x;
+    ws.next_b = blockIdx.y;
+    ws.phase = 0;
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"((unsigned)__cvta_generic_to_shared(&ws.bar))
+                 : "memory");
+  }
+}
+
+/* one thread: ask for the next logical CTA (thread 0 read the response buffer before the last barrier) */
+__device__ __forceinline__ void steal_request(WorkSteal& ws) {
+  const unsigned resp = (unsigned)__cvta_generic_to_shared(ws.response);
+  const unsigned bar = (unsigned)__cvta_generic_to_shared(&ws.bar);
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  asm volatile("clusterlaunchcontrol.try_cancel.async.shared::cta.mbarrier::complete_tx::bytes.b128 [%0], [%1];"
+               ::"r"(resp), "r"(bar) : "memory");
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], 16;" ::"r"(bar) : "memory");
+}
+
+/* thread 0: wait for the answer and publish the next item (next_g = -1: none, or nothing was asked) */
+__device__ __forceinline__ void steal_next(WorkSteal& ws) {
+  if (!ws.requested) {
+    ws.next_g = -1;
+    return;
+  }
+  const unsigned bar = (unsigned)__cvta_generic_to_shared(&ws.bar);
+  unsigned done = 0;
+  do {
+    asm volatile("{\n\t.reg .pred p;\n\t"
+                 "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+                 "selp.u32 %0, 1, 0, p;\n\t}"
+                 : "=r"(done) : "r"(bar), "r"(ws.phase) : "memory");
+  } while (!done);
+  ws.phase ^= 1u;
+  unsigned long long lo, hi;
+  asm volatile("ld.shared.v2.b64 {%0, %1}, [%2];"
+               : "=l"(lo), "=l"(hi) : "r"((unsigned)__cvta_generic_to_shared(ws.response)) : "memory");
+  unsigned ok = 0;
+  asm volatile("{\n\t.reg .b128 q;\n\t.reg .pred p;\n\t"
+               "mov.b128 q, {%1, %2};\n\t"
+               "clusterlaunchcontrol.query_cancel.is_canceled.pred.b128 p, q;\n\t"
+               "selp.u32 %0, 1, 0, p;\n\t}"
+               : "=r"(ok)
+               : "l"(lo), "l"(hi));
+  if (!ok) {
+    ws.next_g = -1;
+    return;
+  }
+  unsigned x, y;
+  asm volatile("{\n\t.reg .b128 q;\n\t"
+               "mov.b128 q, {%2, %3};\n\t"
+               "clusterlaunchcontrol.query_cancel.get_first_ctaid.v4.b32.b128 {%0, %1, _, _}, q;\n\t}"
+               : "=r"(x), "=r"(y)
+               : "l"(lo), "l"(hi));
+  ws.next_g = (int)x;
+  ws.next_b = (int)y;
 }
 
 template <int RT>
@@ -490,183 +590,203 @@ sdfr_forward_kernel(const __grid_constant__ FwdParams P) {
   MomentAcc& acc_s = *reinterpret_cast<MomentAcc*>(acc_mem);
   __shared__ int next_q, n_live;
   __shared__ unsigned worklist[kListCap];
+  __shared__ WorkSteal ws;
 
-  const int b = blockIdx.y + P.z_offset;
-  const int g = blockIdx.x, G = gridDim.x;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int lane_x = lane & 7, lane_y = lane >> 3;
-  const int W = P.cam.W, H = P.cam.H;
-  float *colx, *rowy;
-  const Tiling T = cta_prologue(Fs, edges, tables, P.use_tables, P.pose, b, P.cam, colx, rowy);
-  const Frame& F = Fs; /* read-only from here on; the march hoists what it needs */
-  float* __restrict__ out = P.depth + (size_t)b * H * W;
-  const float* __restrict__ grid = P.sdf + (size_t)b * P.sdf_stride;
-  const float* __restrict__ obs_img = MODE >= 1 ? P.depth_obs + (size_t)b * P.obs_stride : nullptr;
-  /* keep the per-hypothesis bases in registers: ptxas otherwise re-derives b*stride inside the
-   * march loop to save two registers (profiles/r01a: 8 of 68 loop instructions) */
-  asm volatile("" : "+l"(out));
-  asm volatile("" : "+l"(grid));
+  steal_init(ws);
+  if (P.image_tables) fill_image_tables(tables, P.cam);
+  __syncthreads();
+  /* one logical CTA (g, b) per iteration: blockIdx first, then the CTAs this one cancels */
+  for (;;) {
+    const int b = ws.next_b + P.z_offset;
+    const int g = ws.next_g, G = gridDim.x;
+    if (threadIdx.x == 0) { /* read again from ws after cta_prologue's barrier */
+      ws.g = g;
+      ws.b = b;
+      ws.requested = 0;
+    }
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int lane_x = lane & 7, lane_y = lane >> 3;
+    const int W = P.cam.W, H = P.cam.H;
+    float *colx, *rowy;
+    const Tiling T =
+        cta_prologue(Fs, edges, tables, P.use_tables && !P.image_tables, P.pose, g, b, P.cam, colx, rowy);
+    const Frame& F = Fs; /* read-only from here on; the march hoists what it needs */
+    float* __restrict__ out = P.depth + (size_t)b * H * W;
+    const float* __restrict__ grid = P.sdf + (size_t)b * P.sdf_stride;
+    const float* __restrict__ obs_img = MODE >= 1 ? P.depth_obs + (size_t)b * P.obs_stride : nullptr;
+    /* keep the per-hypothesis bases in registers: ptxas otherwise re-derives b*stride inside the
+     * march loop to save two registers (profiles/r01a: 8 of 68 loop instructions) */
+    asm volatile("" : "+l"(out));
+    asm volatile("" : "+l"(grid));
 
-  /* pass 1: tiles that cannot see the box are zero (cu:294-296 writes 0 for these rays); one
-   * whole 32x8 tile per warp, two 16-byte stores per lane */
-  {
-    const int n_tiles = T.tiles_x * T.tiles_y;
-    const bool vec = ((W & 3) == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
-    for (int t = g + warp * G; t < n_tiles; t += kWarps * G) {
-      const int ty = t / T.tiles_x, tx = t - ty * T.tiles_x;
-      if (tx >= T.rtx0 && tx < T.rtx0 + T.rtw && ty >= T.rty0 && ty < T.rty0 + T.rth) continue;
-      const int x0 = tx * kTileW, y0 = ty * kTileH;
-      if (vec && x0 + kTileW <= W && y0 + kTileH <= H) {
-        float4* p = reinterpret_cast<float4*>(out + (size_t)(y0 + lane_y) * W + x0) + lane_x;
-        const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        p[0] = z4;
-        p[W] = z4; /* 4 rows further down: 4*W floats = W float4 */
-      } else {
-        for (int i = lane; i < kThreads; i += 32) {
-          const int px = x0 + (i & (kTileW - 1)), py = y0 + (i / kTileW);
-          if (px < W && py < H) out[(size_t)py * W + px] = 0.0f;
-        }
-      }
-    }
-  }
-
-  /* pass 2: tiles inside the box's rectangle.  The CTA owns rectangle tiles g, g+G, ...  Their
-   * 8x4-pixel warp tiles are first tested against the box silhouette by single threads (8 half-plane
-   * tests each): the ones that cannot see the box are zero-filled on the spot, the others are
-   * compacted into a shared-memory work list which the warps then drain dynamically (a warp whose
-   * rays finish early takes the next entry).  Testing inside the drain loop instead cost ~90 warp
-   * instructions per culled warp tile and ~50 per live one -- 21 % of all executed instructions at
-   * BASELINE config 2 (profiles/r01g_ncu_fused_segments.txt). */
-  if (MODE == 2 && WANT_POSE) moments_clear(acc_s); /* own column only: no barrier needed */
-  float err_acc = 0.0f, cnt_acc = 0.0f, inl_acc = 0.0f;
-  unsigned st_steps = 0, st_entered = 0, st_hit = 0, st_capped = 0;
-  const int n_rect = T.rtw * T.rth;
-  const int n_cand = n_rect > g ? ((n_rect - g + G - 1) / G) * kWarps : 0;
-  /* compile-time grid constants (immediates) for the common resolutions */
-  const Grid Gc = RT > 0 ? make_grid(RT, LT) : P.grid;
-  const bool vec_ok = ((W & 3) == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
-  for (int c0 = 0; c0 < n_cand; c0 += kListCap) {
-    const int n_here = n_cand - c0 < kListCap ? n_cand - c0 : kListCap;
-    __syncthreads(); /* previous chunk drained; list / counters reusable */
-    if (threadIdx.x == 0) {
-      n_live = 0;
-      next_q = kWarps;
-    }
-    __syncthreads();
-    /* 8 lanes per candidate: lane e tests hull edge e, then stores one float4 of the zero fill */
-    const unsigned grp_mask = 0xffu << (lane & 24);
-    const HullEdge my_edge = edges[lane & 7];
-    const float inv_rtw = 1.0f / (float)(T.rtw > 0 ? T.rtw : 1);
-    for (int i0 = 0; i0 < n_here; i0 += kThreads / 8) {
-      const int i = i0 + (threadIdx.x >> 3);
-      const bool have = i < n_here;
-      const int cand = c0 + (have ? i : 0);
-      const int r = g + (cand >> 3) * G, sub = cand & 7;
-      const int wty = div_by(r, T.rtw, inv_rtw);
-      const int tx = T.rtx0 + (r - wty * T.rtw), ty = T.rty0 + wty;
-      const int wx0 = tx * kTileW + ((sub & 3) << 3), wy0 = ty * kTileH + ((sub >> 2) << 2);
-      const bool out_rect = wx0 >= F.x1 || wx0 + 8 <= F.x0 || wy0 >= F.y1 || wy0 + 4 <= F.y0;
-      const bool edge_out = hull_block_outside(my_edge, (float)wx0, (float)wy0, 8.0f, 4.0f);
-      const bool culled = (__ballot_sync(kFull, edge_out || out_rect) & grp_mask) != 0;
-      if (!have) continue;
-      if (!culled) {
-        if ((lane & 7) == 0)
-          worklist[atomicAdd(&n_live, 1)] = (unsigned)(wx0 >> 3) | ((unsigned)(wy0 >> 2) << 16);
-      } else if (wx0 < W && wy0 < H) { /* cu:294-296 writes 0 for these rays */
-        const int yy = (lane & 7) >> 1, xh = (lane & 1) << 2;
-        if (vec_ok && wx0 + 8 <= W && wy0 + 4 <= H) {
-          *reinterpret_cast<float4*>(out + (size_t)(wy0 + yy) * W + wx0 + xh) =
-              make_float4(0.f, 0.f, 0.f, 0.f);
-        } else if (wy0 + yy < H) {
-          for (int xx = xh; xx < xh + 4 && wx0 + xx < W; ++xx) out[(size_t)(wy0 + yy) * W + wx0 + xx] = 0.0f;
-        }
-      }
-    }
-    __syncthreads();
-    const int n_q = n_live;
-    for (int q = warp; q < n_q;) {
-      const unsigned packed = worklist[q];
-      const int px = (int)((packed & 0xffffu) << 3) + lane_x, py = (int)((packed >> 16) << 2) + lane_y;
-      const bool inimg = px < W && py < H;
-      float z = 0.0f;
-      Ray ray;
-      if (inimg && px >= F.x0 && px < F.x1 && py >= F.y0 && py < F.y1) {
-        const float ux = P.use_tables ? colx[px] : pixel_dx(px, P.cam.cx, P.cam.fx);
-        const float uy = P.use_tables ? rowy[py] : pixel_dy(py, P.cam.cy, P.cam.fy);
-        ray = make_ray(F, ux, uy);
-        float t_min, t_max;
-        if (ray_cull_and_box(F, ray, t_min, t_max)) {
-          int steps;
-          bool capped;
-          z = march<RT, LT>(grid, Gc, F, ray, t_min, t_max, P.threshold, steps, capped);
-          if (STATS) {
-            st_steps += steps;
-            st_entered += 1;
-            st_hit += z != 0.0f;
-            st_capped += capped;
+    /* pass 1: tiles that cannot see the box are zero (cu:294-296 writes 0 for these rays); one
+     * whole 32x8 tile per warp, two 16-byte stores per lane */
+    {
+      const int n_tiles = T.tiles_x * T.tiles_y;
+      const bool vec = ((W & 3) == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
+      for (int t = g + warp * G; t < n_tiles; t += kWarps * G) {
+        const int ty = t / T.tiles_x, tx = t - ty * T.tiles_x;
+        if (tx >= T.rtx0 && tx < T.rtx0 + T.rtw && ty >= T.rty0 && ty < T.rty0 + T.rth) continue;
+        const int x0 = tx * kTileW, y0 = ty * kTileH;
+        if (vec && x0 + kTileW <= W && y0 + kTileH <= H) {
+          float4* p = reinterpret_cast<float4*>(out + (size_t)(y0 + lane_y) * W + x0) + lane_x;
+          const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+          p[0] = z4;
+          p[W] = z4; /* 4 rows further down: 4*W floats = W float4 */
+        } else {
+          for (int i = lane; i < kThreads; i += 32) {
+            const int px = x0 + (i & (kTileW - 1)), py = y0 + (i / kTileW);
+            if (px < W && py < H) out[(size_t)py * W + px] = 0.0f;
           }
         }
       }
-      float sgn = 0.0f; /* MODE 2: sign(est - obs) on overlap pixels, 0 = nothing to back-propagate */
-      if (inimg) {
-        const unsigned pix = (unsigned)py * (unsigned)W + (unsigned)px;
-        out[pix] = z;
-        if (MODE >= 1 && z > 0.0f) {
-          /* masked L1 against the observation (estimation/simple_setup.py:125-131) */
-          const float obs = __ldg(obs_img + pix);
-          if (obs > 0.0f) {
-            err_acc += fabsf(z - obs);
-            cnt_acc += 1.0f;
-            /* result selection (estimation/simple_setup.py:183-185): relative error below the
-             * threshold; IEEE division, the same expression the reference evaluates in torch */
-            if (P.n_inlier) inl_acc += __fdiv_rn(fabsf(obs - z), obs) < P.inlier_threshold ? 1.0f : 0.0f;
-            if (MODE == 2 && z != obs) sgn = z > obs ? 1.0f : -1.0f;
+    }
+
+    /* pass 2: tiles inside the box's rectangle.  The CTA owns rectangle tiles g, g+G, ...  Their
+     * 8x4-pixel warp tiles are first tested against the box silhouette by single threads (8 half-plane
+     * tests each): the ones that cannot see the box are zero-filled on the spot, the others are
+     * compacted into a shared-memory work list which the warps then drain dynamically (a warp whose
+     * rays finish early takes the next entry).  Testing inside the drain loop instead cost ~90 warp
+     * instructions per culled warp tile and ~50 per live one -- 21 % of all executed instructions at
+     * BASELINE config 2 (profiles/r01g_ncu_fused_segments.txt). */
+    if (MODE == 2 && WANT_POSE) moments_clear(acc_s); /* own column only: no barrier needed */
+    float err_acc = 0.0f, cnt_acc = 0.0f, inl_acc = 0.0f;
+    unsigned st_steps = 0, st_entered = 0, st_hit = 0, st_capped = 0;
+    const int n_rect = T.rtw * T.rth;
+    const int n_cand = n_rect > item_g(ws) ? ((n_rect - item_g(ws) + G - 1) / G) * kWarps : 0;
+    /* compile-time grid constants (immediates) for the common resolutions */
+    const Grid Gc = RT > 0 ? make_grid(RT, LT) : P.grid;
+    const bool vec_ok = ((W & 3) == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
+    for (int c0 = 0; c0 < n_cand; c0 += kListCap) {
+      const int n_here = n_cand - c0 < kListCap ? n_cand - c0 : kListCap;
+      __syncthreads(); /* previous chunk drained; list / counters reusable */
+      if (threadIdx.x == 0) {
+        n_live = 0;
+        next_q = kWarps;
+      }
+      __syncthreads();
+      /* 8 lanes per candidate: lane e tests hull edge e, then stores one float4 of the zero fill */
+      const unsigned grp_mask = 0xffu << (lane & 24);
+      const HullEdge my_edge = edges[lane & 7];
+      const float inv_rtw = 1.0f / (float)(T.rtw > 0 ? T.rtw : 1);
+      for (int i0 = 0; i0 < n_here; i0 += kThreads / 8) {
+        const int i = i0 + (threadIdx.x >> 3);
+        const bool have = i < n_here;
+        const int cand = c0 + (have ? i : 0);
+        const int r = item_g(ws) + (cand >> 3) * G, sub = cand & 7;
+        const int wty = div_by(r, T.rtw, inv_rtw);
+        const int tx = T.rtx0 + (r - wty * T.rtw), ty = T.rty0 + wty;
+        const int wx0 = tx * kTileW + ((sub & 3) << 3), wy0 = ty * kTileH + ((sub >> 2) << 2);
+        const bool out_rect = wx0 >= F.x1 || wx0 + 8 <= F.x0 || wy0 >= F.y1 || wy0 + 4 <= F.y0;
+        const bool edge_out = hull_block_outside(my_edge, (float)wx0, (float)wy0, 8.0f, 4.0f);
+        const bool culled = (__ballot_sync(kFull, edge_out || out_rect) & grp_mask) != 0;
+        if (!have) continue;
+        if (!culled) {
+          if ((lane & 7) == 0)
+            worklist[atomicAdd(&n_live, 1)] = (unsigned)(wx0 >> 3) | ((unsigned)(wy0 >> 2) << 16);
+        } else if (wx0 < W && wy0 < H) { /* cu:294-296 writes 0 for these rays */
+          const int yy = (lane & 7) >> 1, xh = (lane & 1) << 2;
+          if (vec_ok && wx0 + 8 <= W && wy0 + 4 <= H) {
+            *reinterpret_cast<float4*>(out + (size_t)(wy0 + yy) * W + wx0 + xh) =
+                make_float4(0.f, 0.f, 0.f, 0.f);
+          } else if (wy0 + yy < H) {
+            for (int xx = xh; xx < xh + 4 && wx0 + xx < W; ++xx) out[(size_t)(wy0 + yy) * W + wx0 + xx] = 0.0f;
           }
         }
       }
-      if (MODE == 2 && __any_sync(kFull, sgn != 0.0f)) {
-        int base = 0;
-        float w8[8];
-        if (sgn != 0.0f) {
-          float m[kMoments];
-#pragma unroll
-          for (int i = 0; i < kMoments; ++i) m[i] = 0.0f;
-          pixel_backward_moments<RT, WANT_SDF, WANT_POSE, LT>(grid, Gc, F, ray, z, sgn,
-                                                              (P.flags & SDFR_SDF_GRAD_EXACT) != 0, base, w8, m);
-          if (WANT_POSE) moments_add(acc_s, m);
+      __syncthreads();
+      const int n_q = n_live;
+      for (int q = warp; q < n_q;) {
+        const unsigned packed = worklist[q];
+        const int px = (int)((packed & 0xffffu) << 3) + lane_x, py = (int)((packed >> 16) << 2) + lane_y;
+        const bool inimg = px < W && py < H;
+        float z = 0.0f;
+        Ray ray;
+        if (inimg && px >= F.x0 && px < F.x1 && py >= F.y0 && py < F.y1) {
+          const float ux = P.use_tables ? colx[px] : pixel_dx(px, P.cam.cx, P.cam.fx);
+          const float uy = P.use_tables ? rowy[py] : pixel_dy(py, P.cam.cy, P.cam.fy);
+          ray = make_ray(F, ux, uy);
+          float t_min, t_max;
+          if (ray_cull_and_box(F, ray, t_min, t_max)) {
+            int steps;
+            bool capped;
+            z = march<RT, LT>(grid, Gc, F, ray, t_min, t_max, P.threshold, steps, capped);
+            if (STATS) {
+              st_steps += steps;
+              st_entered += 1;
+              st_hit += z != 0.0f;
+              st_capped += capped;
+            }
+          }
         }
-        if (WANT_SDF)
-          scatter_sdf_warp<RT>(P.grad_sdf + (size_t)b * P.grad_sdf_stride, Gc, base, w8, sgn != 0.0f, lane);
+        float sgn = 0.0f; /* MODE 2: sign(est - obs) on overlap pixels, 0 = nothing to back-propagate */
+        if (inimg) {
+          const unsigned pix = (unsigned)py * (unsigned)W + (unsigned)px;
+          out[pix] = z;
+          if (MODE >= 1 && z > 0.0f) {
+            /* masked L1 against the observation (estimation/simple_setup.py:125-131) */
+            const float obs = __ldg(obs_img + pix);
+            if (obs > 0.0f) {
+              err_acc += fabsf(z - obs);
+              cnt_acc += 1.0f;
+              /* result selection (estimation/simple_setup.py:183-185): relative error below the
+               * threshold; IEEE division, the same expression the reference evaluates in torch */
+              if (P.n_inlier) inl_acc += __fdiv_rn(fabsf(obs - z), obs) < P.inlier_threshold ? 1.0f : 0.0f;
+              if (MODE == 2 && z != obs) sgn = z > obs ? 1.0f : -1.0f;
+            }
+          }
+        }
+        if (MODE == 2 && __any_sync(kFull, sgn != 0.0f)) {
+          int base = 0;
+          float w8[8];
+          if (sgn != 0.0f) {
+            float m[kMoments];
+  #pragma unroll
+            for (int i = 0; i < kMoments; ++i) m[i] = 0.0f;
+            pixel_backward_moments<RT, WANT_SDF, WANT_POSE, LT>(grid, Gc, F, ray, z, sgn,
+                                                                (P.flags & SDFR_SDF_GRAD_EXACT) != 0, base, w8, m);
+            if (WANT_POSE) moments_add(acc_s, m);
+          }
+          if (WANT_SDF)
+            scatter_sdf_warp<RT>(P.grad_sdf + (size_t)item_b(ws) * P.grad_sdf_stride, Gc, base, w8, sgn != 0.0f, lane);
+        }
+        if (lane == 0) q = atomicAdd(&next_q, 1);
+        q = __shfl_sync(kFull, q, 0);
       }
-      if (lane == 0) q = atomicAdd(&next_q, 1);
-      q = __shfl_sync(kFull, q, 0);
     }
-  }
+    /* the first warp out of the work list asks for the next logical CTA: late enough that a CTA still
+     * busy with its item does not reserve one that another CTA could start sooner, early enough that
+     * the answer arrives while the other warps finish */
+    if (P.steal && lane == 0 && atomicExch(&ws.requested, 1) == 0) steal_request(ws);
 
-  if (STATS) {
-    const unsigned s = __reduce_add_sync(kFull, st_steps), e = __reduce_add_sync(kFull, st_entered);
-    const unsigned h = __reduce_add_sync(kFull, st_hit), c = __reduce_add_sync(kFull, st_capped);
-    if (lane == 0) {
-      if (s) atomicAdd(P.stats + 0, (unsigned long long)s);
-      if (e) atomicAdd(P.stats + 1, (unsigned long long)e);
-      if (h) atomicAdd(P.stats + 2, (unsigned long long)h);
-      if (c) atomicAdd(P.stats + 3, (unsigned long long)c);
+    if (STATS) {
+      const unsigned s = __reduce_add_sync(kFull, st_steps), e = __reduce_add_sync(kFull, st_entered);
+      const unsigned h = __reduce_add_sync(kFull, st_hit), c = __reduce_add_sync(kFull, st_capped);
+      if (lane == 0) {
+        if (s) atomicAdd(P.stats + 0, (unsigned long long)s);
+        if (e) atomicAdd(P.stats + 1, (unsigned long long)e);
+        if (h) atomicAdd(P.stats + 2, (unsigned long long)h);
+        if (c) atomicAdd(P.stats + 3, (unsigned long long)c);
+      }
     }
+    if (MODE >= 1) {
+      err_acc = warp_sum(err_acc);
+      cnt_acc = warp_sum(cnt_acc);
+      if (lane == 0) {
+        if (err_acc != 0.0f) atomicAdd(P.loss_sum + item_b(ws), err_acc);
+        if (cnt_acc != 0.0f) atomicAdd(P.n_overlap + item_b(ws), cnt_acc);
+      }
+      if (P.n_inlier) {
+        inl_acc = warp_sum(inl_acc);
+        if (lane == 0 && inl_acc != 0.0f) atomicAdd(P.n_inlier + item_b(ws), inl_acc);
+      }
+    }
+    if (MODE == 2 && WANT_POSE)
+      reduce_pose(acc_s, F, Gc, item_b(ws), P.grad_position, P.grad_orientation, P.grad_inv_scale, P.flags);
+    if (threadIdx.x == 0) steal_next(ws);
+    __syncthreads(); /* next item published; Fs, acc_s, ws.g / ws.b and the work list are free again */
+    if (ws.next_g < 0) break;
   }
-  if (MODE >= 1) {
-    err_acc = warp_sum(err_acc);
-    cnt_acc = warp_sum(cnt_acc);
-    if (lane == 0) {
-      if (err_acc != 0.0f) atomicAdd(P.loss_sum + b, err_acc);
-      if (cnt_acc != 0.0f) atomicAdd(P.n_overlap + b, cnt_acc);
-    }
-    if (P.n_inlier) {
-      inl_acc = warp_sum(inl_acc);
-      if (lane == 0 && inl_acc != 0.0f) atomicAdd(P.n_inlier + b, inl_acc);
-    }
-  }
-  if (MODE == 2 && WANT_POSE)
-    reduce_pose(acc_s, F, Gc, b, P.grad_position, P.grad_orientation, P.grad_inv_scale, P.flags);
 }
 
 /* ------------------------------------------------------------------------------------------
@@ -703,7 +823,7 @@ sdfr_backward_kernel(const __grid_constant__ BwdParams P) {
   }
 
   float *colx, *rowy;
-  const Tiling T = cta_prologue(Fs, nullptr, tables, P.use_tables, P.pose, b, P.cam, colx, rowy);
+  const Tiling T = cta_prologue(Fs, nullptr, tables, P.use_tables, P.pose, g, b, P.cam, colx, rowy);
   const Frame& F = Fs;
   const float* __restrict__ depth = P.depth + (size_t)b * H * W;
   const float* __restrict__ upimg =
@@ -1333,10 +1453,17 @@ int launch_forward(FwdParams P, int batch, cudaStream_t s) {
   const size_t smem = table_bytes(P.cam.W, P.cam.H);
   P.use_tables = smem != 0;
   const int G = ctas_per_hypothesis(batch, P.cam.W, P.cam.H);
+  const int n_tiles = ((P.cam.W + kTileW - 1) / kTileW) * ((P.cam.H + kTileH - 1) / kTileH);
   const bool skewed = P.grid.layout == kLayoutSkewed;
   for (int z0 = 0; z0 < batch; z0 += 65535) {
     P.z_offset = z0;
     const dim3 grid(G, batch - z0 < 65535 ? batch - z0 : 65535);
+    /* a launch that fits in one wave has nothing to steal: its CTAs do not wait for a try_cancel
+     * answer.  With one CTA per tile (a single frame) each item fills the 32 + 8 table entries of its
+     * own tile, as without stealing: the whole image's table (1120 double divisions at 640x480)
+     * would lengthen every first-wave CTA of a latency-bound launch. */
+    P.steal = (long long)G * grid.y > (long long)sm_count() * kFwdBlocks;
+    P.image_tables = P.use_tables && P.steal && G < n_tiles;
 #define SDFR_CALL(RT, LT) launch_forward_rt<RT, LT, MODE, STATS>(P, grid, smem, s)
     SDFR_DISPATCH_RT_LT(P.grid.R, skewed, SDFR_CALL);
 #undef SDFR_CALL
