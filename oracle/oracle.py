@@ -160,14 +160,16 @@ def render_composite(sdfs, positions, orientations, inv_scales, width, height, c
 
 def render_composite_backward(grad_depth, depth, winner, sdfs, positions, orientations,
                               inv_scales, width, height, cx, cy, fx, fy,
-                              sdf_grad_mode="reference", dtype=np.float32, nthreads=1):
+                              sdf_grad_mode="reference", dtype=np.float32, nthreads=1,
+                              want_deriv=False):
     """Per-object gradients of a min-depth composite: each pixel back-propagates to its winner."""
     out = []
     for k in range(len(sdfs)):
         dk = np.where(winner == k, depth, 0).astype(dtype)
         out.append(render_backward(grad_depth, dk, sdfs[k], positions[k], orientations[k],
                                    inv_scales[k], width, height, cx, cy, fx, fy,
-                                   sdf_grad_mode=sdf_grad_mode, dtype=dtype, nthreads=nthreads))
+                                   sdf_grad_mode=sdf_grad_mode, dtype=dtype, nthreads=nthreads,
+                                   want_deriv=want_deriv))
     return out
 
 

@@ -1418,21 +1418,23 @@ size_t table_bytes(int W, int H) {
 
 template <int RT, int LT, int MODE, bool STATS>
 void launch_forward_rt(FwdParams& P, dim3 grid, size_t smem, cudaStream_t s) {
-  if (MODE != 2) {
+  /* constexpr: MODE 0 and 1 instantiate their own kernel only -- no launch of theirs can reach the
+   * gradient variants below, and every instantiation is machine code the library ships */
+  if constexpr (MODE != 2) {
     sdfr_forward_kernel<RT, LT, MODE, STATS, false, false><<<grid, kThreads, smem, s>>>(P);
-    return;
+  } else {
+    const bool want_sdf = (P.flags & SDFR_GRAD_SDF) != 0;
+    const bool want_pose =
+        (P.flags & (SDFR_GRAD_POSITION | SDFR_GRAD_ORIENTATION | SDFR_GRAD_INV_SCALE)) != 0;
+    if (want_sdf && want_pose)
+      sdfr_forward_kernel<RT, LT, MODE, STATS, true, true><<<grid, kThreads, smem, s>>>(P);
+    else if (want_sdf)
+      sdfr_forward_kernel<RT, LT, MODE, STATS, true, false><<<grid, kThreads, smem, s>>>(P);
+    else if (want_pose)
+      sdfr_forward_kernel<RT, LT, MODE, STATS, false, true><<<grid, kThreads, smem, s>>>(P);
+    else
+      sdfr_forward_kernel<RT, LT, 1, STATS, false, false><<<grid, kThreads, smem, s>>>(P);
   }
-  const bool want_sdf = (P.flags & SDFR_GRAD_SDF) != 0;
-  const bool want_pose =
-      (P.flags & (SDFR_GRAD_POSITION | SDFR_GRAD_ORIENTATION | SDFR_GRAD_INV_SCALE)) != 0;
-  if (want_sdf && want_pose)
-    sdfr_forward_kernel<RT, LT, MODE, STATS, true, true><<<grid, kThreads, smem, s>>>(P);
-  else if (want_sdf)
-    sdfr_forward_kernel<RT, LT, MODE, STATS, true, false><<<grid, kThreads, smem, s>>>(P);
-  else if (want_pose)
-    sdfr_forward_kernel<RT, LT, MODE, STATS, false, true><<<grid, kThreads, smem, s>>>(P);
-  else
-    sdfr_forward_kernel<RT, LT, 1, STATS, false, false><<<grid, kThreads, smem, s>>>(P);
 }
 
 /* common resolutions get compile-time pitches (immediate-offset gathers) in both layouts; every
